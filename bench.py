@@ -18,6 +18,10 @@ cpu_baseline objects: `ntt_2^24_round_trip` (configs[1]) and `msm_2^20` (configs
           cores; the Rust crate cannot be built here) on a BOUNDED sample of the same shape (smaller k), scaled linearly in the rows.
 
 Every proof timed here is checked AFTER the timed region by the pinned oracle verifier (`verified`), never inside it.
+
+  --dump-outputs DIR   after the timed steps, the proof bytes of the last timed step of each witness placement as
+          DIR/proof_device_witness.npy and DIR/proof_host_witness.npy (float64, one element per byte; inputs are seeded, so two
+          builds given the same arguments can be compared output for output)
 """
 import argparse
 import json
@@ -351,6 +355,21 @@ def make_provers(sc, pk, pin):
     return (lambda: prove(True)), (lambda: prove(False)), inst
 
 
+def dump_outputs(out_dir, proofs):
+    """--dump-outputs: each proof as <out_dir>/<name>.npy, one float64 per byte (exact)"""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, proof in proofs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.frombuffer(proof, dtype=np.uint8).astype(np.float64))
+
+
+def positive_int(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError(f"must be >= 1, got {v}")
+    return v
+
+
 def time_steps(fn, warmup, steps, barrier):
     for _ in range(warmup):
         fn()
@@ -365,16 +384,19 @@ def time_steps(fn, warmup, steps, barrier):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=positive_int, default=5)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write the last timed step's proofs as DIR/<name>.npy")
     ap.add_argument("--cpu-proof-child", nargs=2, type=int, default=None, help=argparse.SUPPRESS)
     args = ap.parse_args()
     if args.cpu_proof_child:
         return _cpu_proof_child(*args.cpu_proof_child)
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the proofs of the GPU path (--impl ours)")
         return run_reference(args)
 
     import numpy as np
@@ -391,7 +413,7 @@ def main():
     if world > 1:
         ctx.init_comm()
     W = max(3, args.warmup)
-    K = max(1, args.steps)
+    K = args.steps
 
     def barrier():
         if world > 1:
@@ -415,13 +437,15 @@ def main():
     if rank == 0:
         sampler.start()
     ctx.prof_enable(False)
-    sec_dev, _ = time_steps(prove_dev, W, K, barrier)
+    sec_dev, proof_dev = time_steps(prove_dev, W, K, barrier)
     sec_dev = max_over_ranks(sec_dev)
     launches0 = ctx.launch_count
     sec_e2e, proof = time_steps(prove_host, 1, K, barrier)
     sec_e2e = max_over_ranks(sec_e2e)
     launches = (ctx.launch_count - launches0) // K
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"proof_device_witness": proof_dev, "proof_host_witness": proof})
     # per-kernel-class device time of ONE more proof (event pairs on the launching stream; outside the timed region because the
     # extra event records would perturb it)
     ctx.prof_enable(True)
@@ -718,4 +742,5 @@ def bench_msm_sharded(ctx, A, world, rank):
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True      # the source tree may be read-only: nothing (not even __pycache__) is written there
     main()

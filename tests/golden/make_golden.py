@@ -1,20 +1,19 @@
 """Extract golden vectors for the hot path from the reference's own fixture.
 
-Run in the build container (needs /root/reference):  python tests/golden/make_golden.py
+Run against a checkout of scroll-tech/zkevm-circuits:  python tests/golden/make_golden.py <zkevm-circuits checkout>
 Source: aggregator/data/batch-task.json -> chunk_proofs[0]  (used by the reference's tests at
 aggregator/src/tests/aggregation.rs:160,244).  It is a genuine SHPLONK proof of the k=25 thin
 compression circuit together with its vk and snark-verifier Protocol.  We keep only what pins the
 encodings/constants of the MSM/NTT path (SURVEY.md 8c): Montgomery limb form, domain generators,
 G1 compression, proof layout, evaluation order, transcript_repr and PARAMS_G2_SECRET_POWER.
 """
-import base64, json, os, re
+import base64, json, os, re, sys
 
-REF = "/root/reference"
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 
-def main():
-    d = json.load(open(f"{REF}/aggregator/data/batch-task.json"))
+def main(ref):
+    d = json.load(open(f"{ref}/aggregator/data/batch-task.json"))
     c = d["chunk_proofs"][0]
     pr = json.loads(base64.b64decode(c["protocol"]))
     out = {
@@ -50,7 +49,7 @@ def main():
                 walk(v)
     walk(pr["quotient"]["numerator"])
     out["numerator_constants_mont_limbs"] = consts
-    src = open(f"{REF}/prover/src/utils.rs").read()
+    src = open(f"{ref}/prover/src/utils.rs").read()
     m = re.search(r'PARAMS_G2_SECRET_POWER: &str = "(.*)";', src)
     out["params_g2_secret_power"] = m.group(1)
     with open(os.path.join(HERE, "thin_chunk_proof.json"), "w") as f:
@@ -59,4 +58,6 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    if len(sys.argv) != 2:
+        sys.exit("usage: python tests/golden/make_golden.py <zkevm-circuits checkout>")
+    main(sys.argv[1])

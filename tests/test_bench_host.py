@@ -28,6 +28,19 @@ def test_cpu_proof_child_runs_in_its_own_process():
     assert rec["k"] == 8 and len(rec["times"]) == 1 and rec["times"][0] > 0 and rec["cores"] >= 1
 
 
+def test_dump_outputs_and_steps_argument(tmp_path):
+    import numpy as np
+    import bench
+    proofs = {"proof_device_witness": bytes(range(256)) * 3, "proof_host_witness": b"\x00\xff\x07"}
+    bench.dump_outputs(str(tmp_path / "out"), proofs)
+    for name, proof in proofs.items():
+        a = np.load(tmp_path / "out" / f"{name}.npy")
+        assert a.dtype == np.float64 and bytes(a.astype(np.uint8)) == proof
+    assert bench.positive_int("3") == 3
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True, timeout=120)
+    assert out.returncode == 2 and "--steps" in out.stderr
+
+
 def test_oracle_thread_count_is_explicit():
     sys.path.insert(0, os.path.join(ROOT, "oracle"))
     import oracle_lib
