@@ -10,7 +10,7 @@ if [ -n "$NCU_MSM" ]; then timeout 300 ncu --set full --clock-control none --imp
 if [ -n "$MULTI" ]; then timeout ${MULTI_TIMEOUT:-300} python -m torch.distributed.run --nnodes=1 --nproc-per-node $MULTI --master-addr 127.0.0.1 --master-port 29517 scripts/multi_gpu_check.py ${MULTI_ARGS} > gpurun_out/${T}_multi.log 2>&1; echo "multi rc=$?"; tail -3 gpurun_out/${T}_multi.log | cut -c1-2500; fi
 if [ -n "$MULTI_BENCH" ]; then ZKB_TRACE=${ZKB_TRACE} timeout ${MBENCH_TIMEOUT:-600} python -m torch.distributed.run --nnodes=1 --nproc-per-node $MULTI_BENCH --master-addr 127.0.0.1 --master-port 29519 bench.py --gpus $MULTI_BENCH --steps 3 --warmup 3 > gpurun_out/${T}_mbench.log 2> gpurun_out/${T}_mbench.err; echo "mbench rc=$?"; tail -1 gpurun_out/${T}_mbench.log | cut -c1-3000; grep -v "^W0\|^\*\*\*\|^$" gpurun_out/${T}_mbench.err | tail -40; fi
 if [ -n "$TRACE_VARIANTS" ]; then
-  for v in "default" "ZKB_NTT_MAX_A=8" "ZKB_MSM_SHIFT_GB=0" "ZKB_NO_SELECTOR_FOLD=1"; do
+  for v in "default" "ZKB_NTT_MAX_A=8" "ZKB_MSM_SHIFT_GB=0"; do
     echo "== $v" >> gpurun_out/${T}_variants.log
     if [ "$v" = "default" ]; then timeout 300 python scripts/proof_trace.py super 20 128 >> gpurun_out/${T}_variants.log 2>&1; else env $v timeout 300 python scripts/proof_trace.py super 20 128 >> gpurun_out/${T}_variants.log 2>&1; fi
   done

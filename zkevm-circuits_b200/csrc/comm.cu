@@ -77,6 +77,18 @@ int32_t comm_allgather(zkb_ctx *ctx, const void *send, void *recv, size_t bytes_
     return ZKB_OK;
 }
 
+int32_t comm_allgather_host(zkb_ctx *ctx, void *host, size_t bytes_per_rank, cudaStream_t st) {
+    if (ctx->nranks <= 1) return ZKB_OK;
+    uint8_t *d = nullptr;
+    const size_t own = (size_t)ctx->rank * bytes_per_rank;
+    ZKB_TRY(scratch_get(ctx, SCR_COMM, (size_t)ctx->nranks * bytes_per_rank, (void **)&d));
+    ZKB_CUDA(cudaMemcpyAsync(d + own, (const uint8_t *)host + own, bytes_per_rank, cudaMemcpyHostToDevice, st));
+    ZKB_TRY(comm_allgather(ctx, d + own, d, bytes_per_rank, st));
+    ZKB_CUDA(cudaMemcpyAsync(host, d, (size_t)ctx->nranks * bytes_per_rank, cudaMemcpyDeviceToHost, st));
+    ZKB_CUDA(cudaStreamSynchronize(st));
+    return ZKB_OK;
+}
+
 int32_t comm_alltoall(zkb_ctx *ctx, const void *send, void *recv, size_t bytes_per_block, cudaStream_t st) {
     if (ctx->nranks <= 1) {
         if (send != recv) ZKB_CUDA(cudaMemcpyAsync(recv, send, bytes_per_block, cudaMemcpyDeviceToDevice, st));
@@ -118,16 +130,9 @@ int32_t comm_window(zkb_ctx *ctx, size_t bytes, cudaStream_t st) {
     ctx->win_bytes = want;
     ctx->win_peers[ctx->rank] = ctx->win_local;
     if (ctx->nranks <= 1) return ZKB_OK;
-    cudaIpcMemHandle_t mine;
-    ZKB_CUDA(cudaIpcGetMemHandle(&mine, ctx->win_local));
-    static_assert(sizeof(cudaIpcMemHandle_t) == 64, "cudaIpcMemHandle_t is 64 bytes");
-    uint8_t *d_h = nullptr;
-    ZKB_TRY(scratch_get(ctx, SCR_COMM, 64 * 16, (void **)&d_h));
-    ZKB_CUDA(cudaMemcpyAsync(d_h + 64 * ctx->rank, &mine, 64, cudaMemcpyHostToDevice, st));
-    ZKB_TRY(comm_allgather(ctx, d_h + 64 * ctx->rank, d_h, 64, st));
     cudaIpcMemHandle_t all[16];
-    ZKB_CUDA(cudaMemcpyAsync(all, d_h, 64 * (size_t)ctx->nranks, cudaMemcpyDeviceToHost, st));
-    ZKB_CUDA(cudaStreamSynchronize(st));
+    ZKB_CUDA(cudaIpcGetMemHandle(&all[ctx->rank], ctx->win_local));
+    ZKB_TRY(comm_allgather_host(ctx, all, sizeof(cudaIpcMemHandle_t), st));
     for (int j = 0; j < ctx->nranks; ++j) {
         if (j == ctx->rank) continue;
         ZKB_CUDA(cudaIpcOpenMemHandle(&ctx->win_peers[j], all[j], cudaIpcMemLazyEnablePeerAccess));

@@ -183,6 +183,10 @@ int32_t batch_invert_device(zkb_ctx *ctx, const Fr *a, Fr *out, uint64_t n, cuda
 int32_t comm_allreduce_u64(zkb_ctx *ctx, void *dev_buf, size_t count, cudaStream_t st);
 // all-gather: every rank contributes bytes_per_rank; recv holds nranks blocks in rank order (send may be recv + rank * bytes_per_rank)
 int32_t comm_allgather(zkb_ctx *ctx, const void *send, void *recv, size_t bytes_per_rank, cudaStream_t st);
+// the same for small HOST buffers: host holds nranks blocks, this rank's block goes out, all come back; synchronises
+int32_t comm_allgather_host(zkb_ctx *ctx, void *host, size_t bytes_per_rank, cudaStream_t st);
+// point-range sharded MSM (cross.cu): every rank passes its own slice of scalars and bases; the full sum lands on every rank's host
+int32_t msm_g1_sharded(zkb_ctx *ctx, const Fr *scalars, const G1Affine *bases, uint64_t n_local, G1Affine *out_host, cudaStream_t st);
 // all-to-all: block s of `send` (bytes_per_block each) goes to rank s; block j of `recv` came from rank j
 int32_t comm_alltoall(zkb_ctx *ctx, const void *send, void *recv, size_t bytes_per_block, cudaStream_t st);
 // stream-ordered barrier across the ranks (a 8-byte all-reduce): work queued before it on every rank is complete when it completes

@@ -297,26 +297,24 @@ extern "C" int32_t zkb_ntt_fr_sharded_dev(zkb_ctx *ctx, const uint64_t *in_dev, 
     return ZKB_OK;
 }
 
+namespace zkb {
 // point-range sharded MSM: this rank's slice -> local Pippenger -> all-gather of the 64-byte partial sums -> host add.
 // Identical result on every rank.  No point crosses NVLink (SURVEY 8e).
+int32_t msm_g1_sharded(zkb_ctx *ctx, const Fr *scalars, const G1Affine *bases, uint64_t n_local, G1Affine *out_host, cudaStream_t st) {
+    G1Affine all[16];
+    ZKB_TRY(msm_g1_device(ctx, scalars, bases, n_local, &all[ctx->rank], st));
+    ZKB_TRY(comm_allgather_host(ctx, all, sizeof(G1Affine), st));
+    return zkb_g1_sum_affine_host((const uint64_t *)all, (uint64_t)ctx->nranks, (uint64_t *)out_host, nullptr);
+}
+}  // namespace zkb
+
 extern "C" int32_t zkb_msm_g1_sharded_dev(zkb_ctx *ctx, const uint64_t *scalars_shard_dev, const uint64_t *bases_shard_dev, uint64_t n_local,
                                           uint64_t out_affine[8], uint8_t *out_compressed, void *stream) {
     ZKB_ARG(ctx && out_affine && (n_local == 0 || (scalars_shard_dev && bases_shard_dev)));
     ZKB_CUDA(cudaSetDevice(ctx->device));
-    cudaStream_t st = pick_stream(ctx, stream);
-    G1Affine part;
-    ZKB_TRY(msm_g1_device(ctx, (const Fr *)scalars_shard_dev, (const G1Affine *)bases_shard_dev, n_local, &part, st));
-    const int P = ctx->nranks;
-    G1Affine all[16];
-    if (P > 1) {
-        G1Affine *d = nullptr;
-        ZKB_TRY(scratch_get(ctx, SCR_COMM, 64 * 16, (void **)&d));
-        ZKB_CUDA(cudaMemcpyAsync(d + ctx->rank, &part, 64, cudaMemcpyHostToDevice, st));
-        ZKB_TRY(comm_allgather(ctx, d + ctx->rank, d, 64, st));
-        ZKB_CUDA(cudaMemcpyAsync(all, d, 64 * (size_t)P, cudaMemcpyDeviceToHost, st));
-        ZKB_CUDA(cudaStreamSynchronize(st));
-    } else {
-        all[0] = part;
-    }
-    return zkb_g1_sum_affine_host((const uint64_t *)all, (uint64_t)P, out_affine, out_compressed);
+    G1Affine r;
+    ZKB_TRY(msm_g1_sharded(ctx, (const Fr *)scalars_shard_dev, (const G1Affine *)bases_shard_dev, n_local, &r, pick_stream(ctx, stream)));
+    memcpy(out_affine, &r, 64);
+    if (out_compressed) g1_compress(r, out_compressed);
+    return ZKB_OK;
 }

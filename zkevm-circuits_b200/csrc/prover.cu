@@ -179,55 +179,12 @@ static bool fr_less(const Fr &a, const Fr &b) {  // halo2curves Ord: canonical i
     return false;
 }
 static Fr fr_pow_i64(const Fr &base, const Fr &base_inv, int64_t e) { return e >= 0 ? fp_pow_u64(base, (uint64_t)e) : fp_pow_u64(base_inv, (uint64_t)(-e)); }
-
-}  // namespace zkb
-using namespace zkb;
-
-struct zkb_pk {
-    zkb_ctx *ctx = nullptr;
-    Csf cs;
-    uint32_t k = 0, ext_k = 0, E = 0, qdeg = 0, chunk = 0, nsets = 0;
-    uint64_t n = 0, N = 0;
-    Fr omega, omega_inv, ext_omega, ext_omega_inv, n_inv, N_inv, zeta;
-    std::vector<Fr> t_inv;
-    DevPool pool;
-    std::vector<Fr *> fixed_values, fixed_polys, sigma_values, sigma_polys;
-    Fr *l0_poly = nullptr, *llast_poly = nullptr, *lblind_poly = nullptr, *xid_poly = nullptr, *omega_pows = nullptr;
-    zkb_srs *srs = nullptr;       // shared ParamsKZG handle (owned when the pk was made by the legacy zkb_pk_create)
-    bool owns_srs = false;
-    G1Affine *g = nullptr, *g_lagrange = nullptr;   // = srs->g / srs->g_lagrange
-    // coset evaluations of the proof-independent polynomials (fixed, sigma, l_0, l_last, l_blind, X) for every coset part,
-    // like upstream's pk.fixed_cosets / permutation cosets / l0 / l_last / l_active_row: [part][poly] -> n elements
-    std::vector<std::vector<Fr *>> coset_cache;
-    // window-shifted copies of the SRS (copy w = 2^(c w) * P_i) for the Pippenger variant with one bucket set per column (= srs->*_shift)
-    G1Affine *g_shift = nullptr, *g_lagrange_shift = nullptr;
-    ~zkb_pk() {
-        if (owns_srs && srs) zkb_srs_destroy(srs);
-    }
-};
-
-struct zkb_session {
-    zkb_pk *pk = nullptr;
-    // 0: Blake2bWrite<_, G1Affine, Challenge255<_>> (benches), 1: snark-verifier-sdk PoseidonTranscript (gen_snark_shplonk),
-    // 2: snark-verifier EvmTranscript over Keccak-256 (gen_evm_proof_shplonk), 3: the CALLER's transcript through zkb_transcript_vtable
-    // (create_proof's generic `T: TranscriptWrite`: the shim forwards the four operations to the Rust object it was handed)
-    int tkind = 0;
-    zkb_transcript_vtable vt{};
-    int32_t cb_error = 0;   // first non-zero return of a caller callback (checked after every stage)
-    Blake2b tr{"Halo2-Transcript"};
-    PoseidonSponge pos;
-    std::vector<uint8_t> evm_buf;
-    std::vector<uint8_t> proof;
-    DevPool pool;
-    std::vector<Fr *> inst_values, inst_polys, adv_values;
-    // columns handed over ahead of their phase (zkb_prove_upload_advice): staged device copies, consumed by zkb_prove_advice_phase
-    std::map<uint32_t, Fr *> early_cols;
-    std::vector<Fr> challenges;
-    uint32_t next_phase = 0;
-    bool finished = false;
-};
-
-namespace zkb {
+// DELTA = 7^(2^28), the generator of the permutation argument's column cosets (permutation/keygen.rs)
+static Fr perm_delta() {
+    Fr delta = fr_from_u64(7);
+    for (int i = 0; i < 28; ++i) delta = fp_sqr(delta);
+    return delta;
+}
 
 // ---------------------------------------------------------------------------------------------------------- transcript
 // base-field coordinate (canonical limbs, < q) -> scalar-field element (x mod r), Montgomery form: snark-verifier's fe_to_fe
@@ -252,105 +209,157 @@ static void push_be32(std::vector<uint8_t> &dst, const F &canonical) {
     const uint8_t *b = (const uint8_t *)canonical.l;
     for (int i = 31; i >= 0; --i) dst.push_back(b[i]);
 }
-static void tr_common_scalar(zkb_session *s, const Fr &v) {
-    if (s->tkind == 3) { const int32_t r = s->vt.common_scalar(s->vt.user, (const uint64_t *)v.l); if (r && !s->cb_error) s->cb_error = r; return; }
-    if (s->tkind == 1) { s->pos.update(v); return; }
-    if (s->tkind == 2) { push_be32(s->evm_buf, fp_to_canonical(v)); return; }
-    const uint8_t pre = 2;
-    Fr c = fp_to_canonical(v);
-    s->tr.update(&pre, 1);
-    s->tr.update(c.l, 32);
-}
-static void tr_write_scalar(zkb_session *s, const Fr &v) {
-    if (s->tkind == 3) { const int32_t r = s->vt.write_scalar(s->vt.user, (const uint64_t *)v.l); if (r && !s->cb_error) s->cb_error = r; return; }
-    tr_common_scalar(s, v);
-    Fr c = fp_to_canonical(v);
-    if (s->tkind == 2) { push_be32(s->proof, c); return; }
-    const uint8_t *b = (const uint8_t *)c.l;
-    s->proof.insert(s->proof.end(), b, b + 32);
-}
-static int32_t tr_write_point(zkb_session *s, const G1Affine &p) {
-    if (p.is_identity()) { set_error("cannot write points at infinity to the transcript"); return ZKB_ERR_STATE; }
-    if (s->tkind == 3) {
-        const int32_t r = s->vt.write_point(s->vt.user, (const uint64_t *)&p);
-        if (r) { set_error("the caller's transcript refused a point (callback returned %d)", r); if (!s->cb_error) s->cb_error = r; return ZKB_ERR_STATE; }
-        return ZKB_OK;
-    }
-    Fq x = fp_to_canonical(p.x), y = fp_to_canonical(p.y);
-    if (s->tkind == 2) {  // absorbed and written uncompressed: x || y, big-endian
-        push_be32(s->evm_buf, x); push_be32(s->evm_buf, y);
-        push_be32(s->proof, x); push_be32(s->proof, y);
-        return ZKB_OK;
-    }
-    if (s->tkind == 1) {
-        s->pos.update(fq_canonical_to_fr(x));
-        s->pos.update(fq_canonical_to_fr(y));
-    } else {
-        const uint8_t pre = 1;
-        s->tr.update(&pre, 1);
-        s->tr.update(x.l, 32);
-        s->tr.update(y.l, 32);
-    }
-    uint8_t comp[32];
-    g1_compress(p, comp);
-    s->proof.insert(s->proof.end(), comp, comp + 32);
-    return ZKB_OK;
-}
-static Fr tr_squeeze(zkb_session *s) {
-    if (s->tkind == 3) {
-        Fr c = Fr::zero();
-        const int32_t r = s->vt.squeeze_challenge(s->vt.user, (uint64_t *)c.l);
-        if (r && !s->cb_error) s->cb_error = r;
-        return c;
-    }
-    if (s->tkind == 1) return s->pos.squeeze();
-    if (s->tkind == 2) {
-        // hash the buffer (plus a 0x01 byte when it holds just the previous digest), keep the digest as the new buffer,
-        // challenge = digest as a big-endian integer mod r
-        if (s->evm_buf.size() == 32) s->evm_buf.push_back(1);
-        uint8_t h[32];
-        keccak256(s->evm_buf.data(), s->evm_buf.size(), h);
-        s->evm_buf.assign(h, h + 32);
-        Fr v;
-        uint8_t *b = (uint8_t *)v.l;
-        for (int i = 0; i < 32; ++i) b[i] = h[31 - i];
-        return fp_mul(v, Fr::r2());  // Montgomery multiply reduces any 256-bit value: v * R^2 / R = v R mod r
-    }
+// Challenge255 of a Blake2b("Halo2-Transcript") state: absorb the 0x00 prefix, then Fr::from_uniform_bytes of the 64-byte
+// digest, (lo + hi * 2^256) mod r, computed with Montgomery multiplications by R^2
+static Fr blake2b_challenge(Blake2b &h) {
     const uint8_t pre = 0;
-    s->tr.update(&pre, 1);
-    uint8_t h[64];
-    s->tr.finalize_copy(h);
+    h.update(&pre, 1);
+    uint8_t d[64];
+    h.finalize_copy(d);
     Fr lo, hi;
-    memcpy(lo.l, h, 32);
-    memcpy(hi.l, h + 32, 32);
-    // Fr::from_uniform_bytes: (lo + hi * 2^256) mod r, computed with Montgomery multiplications by R^2
+    memcpy(lo.l, d, 32);
+    memcpy(hi.l, d + 32, 32);
     const Fr r2 = Fr::r2();
     return fp_add(fp_mul(lo, r2), fp_mul(fp_mul(hi, r2), r2));
 }
+
+// The transcript of one proof.  The kind values are those of the C ABI (zkb_prove_begin_ex, zkb_transcript_script_host).
+enum TranscriptKind : int32_t {
+    TR_BLAKE2B = 0,    // Blake2bWrite<_, G1Affine, Challenge255<_>> (benches)
+    TR_POSEIDON = 1,   // snark-verifier-sdk PoseidonTranscript (gen_snark_shplonk)
+    TR_EVM = 2,        // snark-verifier EvmTranscript over Keccak-256 (gen_evm_proof_shplonk)
+    TR_CALLER = 3,     // the caller's transcript through zkb_transcript_vtable (create_proof's generic `T: TranscriptWrite`: the
+                       // shim forwards the four operations to the Rust object it was handed)
+};
+struct Transcript {
+    TranscriptKind kind = TR_BLAKE2B;
+    zkb_transcript_vtable vt{};
+    int32_t cb_error = 0;   // first non-zero return of a caller callback (checked after every stage)
+    Blake2b blake{"Halo2-Transcript"};
+    PoseidonSponge pos;
+    std::vector<uint8_t> evm_buf;
+    std::vector<uint8_t> proof;
+
+    void callback(int32_t r) {
+        if (r && !cb_error) cb_error = r;
+    }
+    // ZKB_ERR_STATE once a caller callback has failed
+    int32_t status() const {
+        if (!cb_error) return ZKB_OK;
+        set_error("the caller's transcript callback failed (%d)", cb_error);
+        return ZKB_ERR_STATE;
+    }
+    void common_scalar(const Fr &v) {
+        if (kind == TR_CALLER) { callback(vt.common_scalar(vt.user, (const uint64_t *)v.l)); return; }
+        if (kind == TR_POSEIDON) { pos.update(v); return; }
+        if (kind == TR_EVM) { push_be32(evm_buf, fp_to_canonical(v)); return; }
+        const uint8_t pre = 2;
+        Fr c = fp_to_canonical(v);
+        blake.update(&pre, 1);
+        blake.update(c.l, 32);
+    }
+    void write_scalar(const Fr &v) {
+        if (kind == TR_CALLER) { callback(vt.write_scalar(vt.user, (const uint64_t *)v.l)); return; }
+        common_scalar(v);
+        Fr c = fp_to_canonical(v);
+        if (kind == TR_EVM) { push_be32(proof, c); return; }
+        const uint8_t *b = (const uint8_t *)c.l;
+        proof.insert(proof.end(), b, b + 32);
+    }
+    int32_t write_point(const G1Affine &p) {
+        if (p.is_identity()) { set_error("cannot write points at infinity to the transcript"); return ZKB_ERR_STATE; }
+        if (kind == TR_CALLER) {
+            const int32_t r = vt.write_point(vt.user, (const uint64_t *)&p);
+            if (r) { set_error("the caller's transcript refused a point (callback returned %d)", r); callback(r); return ZKB_ERR_STATE; }
+            return ZKB_OK;
+        }
+        Fq x = fp_to_canonical(p.x), y = fp_to_canonical(p.y);
+        if (kind == TR_EVM) {  // absorbed and written uncompressed: x || y, big-endian
+            push_be32(evm_buf, x); push_be32(evm_buf, y);
+            push_be32(proof, x); push_be32(proof, y);
+            return ZKB_OK;
+        }
+        if (kind == TR_POSEIDON) {
+            pos.update(fq_canonical_to_fr(x));
+            pos.update(fq_canonical_to_fr(y));
+        } else {
+            const uint8_t pre = 1;
+            blake.update(&pre, 1);
+            blake.update(x.l, 32);
+            blake.update(y.l, 32);
+        }
+        uint8_t comp[32];
+        g1_compress(p, comp);
+        proof.insert(proof.end(), comp, comp + 32);
+        return ZKB_OK;
+    }
+    Fr squeeze() {
+        if (kind == TR_CALLER) {
+            Fr c = Fr::zero();
+            callback(vt.squeeze_challenge(vt.user, (uint64_t *)c.l));
+            return c;
+        }
+        if (kind == TR_POSEIDON) return pos.squeeze();
+        if (kind == TR_EVM) {
+            // hash the buffer (plus a 0x01 byte when it holds just the previous digest), keep the digest as the new buffer,
+            // challenge = digest as a big-endian integer mod r
+            if (evm_buf.size() == 32) evm_buf.push_back(1);
+            uint8_t h[32];
+            keccak256(evm_buf.data(), evm_buf.size(), h);
+            evm_buf.assign(h, h + 32);
+            Fr v;
+            uint8_t *b = (uint8_t *)v.l;
+            for (int i = 0; i < 32; ++i) b[i] = h[31 - i];
+            return fp_mul(v, Fr::r2());  // Montgomery multiply reduces any 256-bit value: v * R^2 / R = v R mod r
+        }
+        return blake2b_challenge(blake);
+    }
+};
+
+}  // namespace zkb
+using namespace zkb;
+
+struct zkb_pk {
+    zkb_ctx *ctx = nullptr;
+    Csf cs;
+    uint32_t k = 0, ext_k = 0, E = 0, qdeg = 0, chunk = 0, nsets = 0;
+    uint64_t n = 0, N = 0;
+    Fr omega, omega_inv, ext_omega, ext_omega_inv, n_inv, N_inv, zeta;
+    std::vector<Fr> t_inv;
+    DevPool pool;
+    std::vector<Fr *> fixed_values, fixed_polys, sigma_values, sigma_polys;
+    Fr *l0_poly = nullptr, *llast_poly = nullptr, *lblind_poly = nullptr, *xid_poly = nullptr, *omega_pows = nullptr;
+    zkb_srs *srs = nullptr;       // shared ParamsKZG handle (owned when the pk was made by the legacy zkb_pk_create)
+    bool owns_srs = false;
+    // coset evaluations of the proof-independent polynomials (fixed, sigma, l_0, l_last, l_blind, X) for every coset part,
+    // like upstream's pk.fixed_cosets / permutation cosets / l0 / l_last / l_active_row: [part][poly] -> n elements
+    std::vector<std::vector<Fr *>> coset_cache;
+    ~zkb_pk() {
+        if (owns_srs && srs) zkb_srs_destroy(srs);
+    }
+};
+
+struct zkb_session {
+    zkb_pk *pk = nullptr;
+    Transcript tr;
+    DevPool pool;
+    std::vector<Fr *> inst_values, inst_polys, adv_values;
+    // columns handed over ahead of their phase (zkb_prove_upload_advice): staged device copies, consumed by zkb_prove_advice_phase
+    std::map<uint32_t, Fr *> early_cols;
+    std::vector<Fr> challenges;
+    uint32_t next_phase = 0;
+    bool finished = false;
+};
+
+namespace zkb {
 
 // ---------------------------------------------------------------------------------------------------------- basis changes
 static int32_t lagrange_to_coeff(zkb_pk *pk, const Fr *values, Fr *poly, cudaStream_t st) {
     return ntt_fr_device(pk->ctx, values, poly, pk->k, pk->omega_inv, &pk->n_inv, 0, nullptr, st);
 }
-static int32_t commit(zkb_pk *pk, const Fr *scalars, const G1Affine *bases, uint64_t len, G1Affine *out, cudaStream_t st) {
-    return msm_g1_device(pk->ctx, scalars, bases, len, out, st);
-}
+// generator of coset part j of the extended domain: zeta * omega_ext^j
+static Fr coset_gen(const zkb_pk *pk, uint32_t j) { return fp_mul(pk->zeta, fp_pow_u64(pk->ext_omega, j)); }
 
-// commit several columns against the same bases with batched MSMs (one pass per <= msm_max_batch columns)
-static int32_t commit_many_local(zkb_pk *pk, const std::vector<Fr *> &cols, const G1Affine *bases, uint64_t len, std::vector<G1Affine> &out, cudaStream_t st) {
-    out.resize(cols.size());
-    const uint32_t maxb = msm_max_batch(len);
-    const G1Affine *shift = (bases == pk->g) ? pk->g_shift : (bases == pk->g_lagrange) ? pk->g_lagrange_shift : nullptr;
-    if (len != pk->n) shift = nullptr;
-    for (size_t done = 0; done < cols.size(); done += maxb) {
-        const uint32_t cur = (uint32_t)std::min<size_t>(maxb, cols.size() - done);
-        const Fr **d_tbl = nullptr;
-        ZKB_TRY(scratch_get(pk->ctx, SCR_MSM_TBL, 64 * sizeof(Fr *), (void **)&d_tbl));
-        ZKB_CUDA(cudaMemcpyAsync(d_tbl, cols.data() + done, cur * sizeof(Fr *), cudaMemcpyHostToDevice, st));
-        ZKB_TRY(msm_g1_batch_device_ex(pk->ctx, d_tbl, cur, shift ? shift : bases, len, out.data() + done, shift != nullptr, st));
-    }
-    return ZKB_OK;
-}
 // multi-GPU dealing of independent units (columns, lookup arguments, coset parts): the `count` units are cut into P contiguous
 // blocks of blk = ceil(count / P), rank r computes block r.  Results live in a slab of P * blk unit slots (the tail of the last
 // blocks is padding), so ONE in-place ncclAllGather (every rank contributes its own block, 1/P of the slab) completes it -- no
@@ -365,49 +374,46 @@ struct Deal {
     }
     bool mine(size_t i) const { return !on || (int)(i / blk) == rank; }
     size_t padded() const { return on ? (size_t)P * blk : count; }
+    size_t first() const { return on ? (size_t)rank * blk : 0; }   // index of this rank's first unit
 };
 static int32_t deal_gather(zkb_ctx *ctx, const Deal &d, void *slab, size_t unit_bytes, cudaStream_t st) {
     if (!d.on) return ZKB_OK;
-    return comm_allgather(ctx, (const uint8_t *)slab + (size_t)d.rank * d.blk * unit_bytes, slab, d.blk * unit_bytes, st);
+    return comm_allgather(ctx, (const uint8_t *)slab + d.first() * unit_bytes, slab, d.blk * unit_bytes, st);
+}
+// the same for a slab of small values on the host (padded() units of unit_bytes; synchronises)
+static int32_t deal_gather_host(zkb_ctx *ctx, const Deal &d, void *slab, size_t unit_bytes, cudaStream_t st) {
+    if (!d.on) return ZKB_OK;
+    return comm_allgather_host(ctx, slab, d.blk * unit_bytes, st);
 }
 
-// commit several columns against the same bases with batched MSMs.  With a communicator the columns are dealt in contiguous blocks
-// (Deal) and the 64-byte results are all-gathered.
-static int32_t commit_many(zkb_pk *pk, const std::vector<Fr *> &cols, const G1Affine *bases, uint64_t len, std::vector<G1Affine> &out, cudaStream_t st) {
+enum { BASIS_G = 0, BASIS_LAGRANGE = 1 };   // the bases of srs_commit_many
+// commit several columns of n scalars against one basis of the SRS with batched MSMs.  With a communicator the columns
+// are dealt in contiguous blocks (Deal) and the 64-byte results are all-gathered; a single commitment (random polynomial, SHPLONK's
+// h and the final quotient) cannot be dealt: it is sharded by point range instead (SURVEY 8e).
+static int32_t commit_many(zkb_pk *pk, int basis, const std::vector<Fr *> &cols, std::vector<G1Affine> &out, cudaStream_t st) {
     zkb_ctx *ctx = pk->ctx;
-    if (ctx->nranks > 1 && cols.size() == 1 && len >= (1u << 14)) {
-        // a single commitment (random polynomial, SHPLONK's h and the final quotient) cannot be dealt: shard it by point range instead
-        // (SURVEY 8e): every rank reduces len / P points, the 64-byte partial sums are all-gathered and added on the host
-        const uint64_t P = (uint64_t)ctx->nranks, lo = len * (uint64_t)ctx->rank / P, hi = len * ((uint64_t)ctx->rank + 1) / P;
-        G1Affine part;
-        ZKB_TRY(msm_g1_device(ctx, cols[0] + lo, bases + lo, hi - lo, &part, st));
-        G1Affine *d_buf = nullptr;
-        ZKB_TRY(scratch_get(ctx, SCR_COMM, 16 * sizeof(G1Affine), (void **)&d_buf));
-        ZKB_CUDA(cudaMemcpyAsync(d_buf + ctx->rank, &part, sizeof(G1Affine), cudaMemcpyHostToDevice, st));
-        ZKB_TRY(comm_allgather(ctx, d_buf + ctx->rank, d_buf, sizeof(G1Affine), st));
-        G1Affine all[16];
-        ZKB_CUDA(cudaMemcpyAsync(all, d_buf, P * sizeof(G1Affine), cudaMemcpyDeviceToHost, st));
-        ZKB_CUDA(cudaStreamSynchronize(st));
-        G1Xyzz acc = G1Xyzz::identity();
-        for (uint64_t r = 0; r < P; ++r) g1_add_mixed(acc, all[r]);
-        out.assign(1, g1_to_affine(acc));
-        return ZKB_OK;
+    const uint64_t n = pk->n;
+    if (ctx->nranks > 1 && cols.size() == 1 && n >= (1u << 14)) {
+        const uint64_t P = (uint64_t)ctx->nranks, lo = n * (uint64_t)ctx->rank / P, hi = n * ((uint64_t)ctx->rank + 1) / P;
+        const G1Affine *bases = basis == BASIS_G ? pk->srs->g : pk->srs->g_lagrange;
+        out.resize(1);
+        return msm_g1_sharded(ctx, cols[0] + lo, bases + lo, hi - lo, out.data(), st);
     }
     const Deal d(ctx, cols.size());
-    if (!d.on) return commit_many_local(pk, cols, bases, len, out, st);
-    std::vector<Fr *> mine;
+    std::vector<const Fr *> mine;
     for (size_t i = 0; i < cols.size(); ++i)
         if (d.mine(i)) mine.push_back(cols[i]);
-    std::vector<G1Affine> part;
-    if (!mine.empty()) ZKB_TRY(commit_many_local(pk, mine, bases, len, part, st));
-    G1Affine *d_buf = nullptr;
-    ZKB_TRY(scratch_get(ctx, SCR_COMM, d.padded() * sizeof(G1Affine), (void **)&d_buf));
-    if (!part.empty()) ZKB_CUDA(cudaMemcpyAsync(d_buf + (size_t)d.rank * d.blk, part.data(), part.size() * sizeof(G1Affine), cudaMemcpyHostToDevice, st));
-    ZKB_TRY(deal_gather(ctx, d, d_buf, sizeof(G1Affine), st));
     out.resize(d.padded());
-    ZKB_CUDA(cudaMemcpyAsync(out.data(), d_buf, d.padded() * sizeof(G1Affine), cudaMemcpyDeviceToHost, st));
-    ZKB_CUDA(cudaStreamSynchronize(st));
+    if (!mine.empty()) ZKB_TRY(srs_commit_many(pk->srs, basis, mine.data(), (uint32_t)mine.size(), n, out.data() + d.first(), st));
+    ZKB_TRY(deal_gather_host(ctx, d, out.data(), sizeof(G1Affine), st));
     out.resize(cols.size());
+    return ZKB_OK;
+}
+// commit_many, then write every commitment to the session's transcript
+static int32_t commit_write(zkb_session *s, int basis, const std::vector<Fr *> &cols, cudaStream_t st) {
+    std::vector<G1Affine> cms;
+    ZKB_TRY(commit_many(s->pk, basis, cols, cms, st));
+    for (auto &cm : cms) ZKB_TRY(s->tr.write_point(cm));
     return ZKB_OK;
 }
 
@@ -463,6 +469,28 @@ static uint32_t compress_exprs(const Csf &cs, const std::vector<uint32_t> &exprs
     for (size_t i = 1; i < exprs.size(); ++i) acc = eb.add(eb.mul(acc, eb.constant(theta)), translate(cs, exprs[i], eb, sm, ch, memo));
     return acc;
 }
+// slot of a permutation column (kind, index) in a table numbered by `sm`
+static uint32_t perm_slot(const SlotMap &sm, const std::array<uint32_t, 2> &c) {
+    return c[0] == N_FIXED ? sm.fixed0 + c[1] : c[0] == N_ADVICE ? sm.advice0 + c[1] : sm.instance0 + c[1];
+}
+
+// upload an interpreter program and its output table, run it over the n rows of the columns in d_cols
+static int32_t run_program(zkb_session *s, const ProgramBuilder &pb, const ExprBuilder &eb, Fr *const *d_cols, const std::vector<Fr *> &outs, cudaStream_t st) {
+    DeviceProgram dp;
+    ZKB_TRY(upload_program(s->pool, pb, eb, dp, st));
+    Fr **d_outs = nullptr;
+    ZKB_TRY(upload_table(s->pool, outs, &d_outs, st));
+    return expr_run_device(s->pk->ctx, dp.code, dp.ncode, dp.nregs, d_cols, dp.consts, d_outs, s->pk->k, 1, 0, st);
+}
+// out (+)= sum_i coefs[i] polys[i] over n coefficients.  Does not synchronise: `coefs` must stay alive until the stream is.
+static int32_t lincomb(zkb_session *s, const std::vector<Fr *> &polys, const std::vector<Fr> &coefs, Fr *out, bool accumulate, cudaStream_t st) {
+    Fr **d_p = nullptr;
+    Fr *d_c = nullptr;
+    ZKB_TRY(upload_table(s->pool, polys, &d_p, st));
+    ZKB_TRY(s->pool.fr(coefs.size(), &d_c));
+    ZKB_CUDA(cudaMemcpyAsync(d_c, coefs.data(), coefs.size() * sizeof(Fr), cudaMemcpyHostToDevice, st));
+    return lincomb_device(s->pk->ctx, d_p, d_c, (uint32_t)polys.size(), s->pk->n, out, accumulate, st);
+}
 
 }  // namespace zkb
 
@@ -505,40 +533,24 @@ static int32_t pk_build(zkb_ctx *ctx, const uint32_t *csf, uint64_t csf_words, c
     pk->N_inv = fp_inv(fr_from_u64(pk->N));
     pk->zeta = host_zeta();
     pk->t_inv.resize(pk->E);
-    for (uint32_t j = 0; j < pk->E; ++j) {
-        Fr gj = fp_mul(pk->zeta, fp_pow_u64(pk->ext_omega, j));
-        pk->t_inv[j] = fp_inv(fp_sub(fp_pow_u64(gj, n), Fr::one()));
-    }
-    pk->g = srs->g;
-    pk->g_lagrange = srs->g_lagrange;
-    pk->g_shift = srs->g_shift;
-    pk->g_lagrange_shift = srs->g_lagrange_shift;
-    // fixed / sigma columns: values and coefficient form
-    auto ingest = [&](const uint64_t *const *src, size_t cnt, std::vector<Fr *> &vals, std::vector<Fr *> &polys) -> int32_t {
+    for (uint32_t j = 0; j < pk->E; ++j) pk->t_inv[j] = fp_inv(fp_sub(fp_pow_u64(coset_gen(pk.get(), j), n), Fr::one()));
+    // fixed / sigma columns (host or device sources): values and coefficient form
+    auto ingest = [&](const void *const *src, size_t cnt, std::vector<Fr *> &vals, std::vector<Fr *> &polys) -> int32_t {
         vals.resize(cnt);
         polys.resize(cnt);
         for (size_t i = 0; i < cnt; ++i) {
             ZKB_TRY(pk->pool.fr(n, &vals[i]));
             ZKB_TRY(pk->pool.fr(n, &polys[i]));
-            ZKB_CUDA(cudaMemcpyAsync(vals[i], src[i], n * sizeof(Fr), cudaMemcpyHostToDevice, st));
+            ZKB_CUDA(cudaMemcpyAsync(vals[i], src[i], n * sizeof(Fr), cudaMemcpyDefault, st));
             ZKB_TRY(lagrange_to_coeff(pk.get(), vals[i], polys[i], st));
         }
         return ZKB_OK;
     };
-    ZKB_TRY(ingest(fixed_values, cs.nf, pk->fixed_values, pk->fixed_polys));
-    if (sigma_dev) {
-        ZKB_ARG(sigma_dev->size() == cs.perm.size());
-        pk->sigma_values.resize(cs.perm.size());
-        pk->sigma_polys.resize(cs.perm.size());
-        for (size_t i = 0; i < cs.perm.size(); ++i) {
-            ZKB_TRY(pk->pool.fr(n, &pk->sigma_values[i]));
-            ZKB_TRY(pk->pool.fr(n, &pk->sigma_polys[i]));
-            ZKB_CUDA(cudaMemcpyAsync(pk->sigma_values[i], (*sigma_dev)[i], n * sizeof(Fr), cudaMemcpyDeviceToDevice, st));
-            ZKB_TRY(lagrange_to_coeff(pk.get(), pk->sigma_values[i], pk->sigma_polys[i], st));
-        }
-    } else {
-        ZKB_TRY(ingest(sigma_values, cs.perm.size(), pk->sigma_values, pk->sigma_polys));
-    }
+    ZKB_TRY(ingest((const void *const *)fixed_values, cs.nf, pk->fixed_values, pk->fixed_polys));
+    ZKB_ARG(!sigma_dev || sigma_dev->size() == cs.perm.size());
+    std::vector<const void *> sigma_src(cs.perm.size());
+    for (size_t i = 0; i < cs.perm.size(); ++i) sigma_src[i] = sigma_dev ? (const void *)(*sigma_dev)[i] : (const void *)sigma_values[i];
+    ZKB_TRY(ingest(sigma_src.data(), cs.perm.size(), pk->sigma_values, pk->sigma_polys));
     // l_0, l_last, l_blind (Lagrange indicator vectors -> coefficient form), X (identity polynomial), omega^i
     ZKB_TRY(pk->pool.fr(n, &pk->l0_poly));
     ZKB_TRY(pk->pool.fr(n, &pk->llast_poly));
@@ -572,8 +584,7 @@ static int32_t pk_build(zkb_ctx *ctx, const uint32_t *csf, uint64_t csf_words, c
             ZKB_TRY(pk->pool.fr(n, &pows));
             pk->coset_cache.resize(pk->E);
             for (uint32_t j = 0; j < pk->E; ++j) {
-                const Fr gj = fp_mul(pk->zeta, fp_pow_u64(pk->ext_omega, j));
-                ZKB_TRY(fr_powers_device(ctx, gj, n, pows, st));
+                ZKB_TRY(fr_powers_device(ctx, coset_gen(pk.get(), j), n, pows, st));
                 pk->coset_cache[j].resize(stat.size());
                 for (size_t i = 0; i < stat.size(); ++i) {
                     ZKB_TRY(pk->pool.fr(n, &pk->coset_cache[j][i]));
@@ -657,9 +668,7 @@ extern "C" int32_t zkb_keygen_pk(zkb_ctx *ctx, const uint32_t *csf, uint64_t csf
     ZKB_CUDA(cudaMemcpyAsync(d_mr, map_row.data(), P * n * 4, cudaMemcpyHostToDevice, st));
     Fr omega = host_root_of_unity(cs.k);
     ZKB_TRY(fr_powers_device(ctx, omega, n, d_om, st));
-    Fr delta = fr_from_u64(7);
-    for (int i = 0; i < 28; ++i) delta = fp_sqr(delta);   // DELTA = 7^(2^28)
-    ZKB_TRY(fr_powers_device(ctx, delta, P + 1, d_dl, st));
+    ZKB_TRY(fr_powers_device(ctx, perm_delta(), P + 1, d_dl, st));
     std::vector<Fr *> sig(P);
     for (size_t c = 0; c < P; ++c) {
         ZKB_TRY(tmp.fr(n, &sig[c]));
@@ -699,9 +708,9 @@ extern "C" int32_t zkb_poseidon_hash_host(const uint64_t *inputs, uint64_t n, ui
 // framing of every transcript kind against the oracle's transcripts.
 extern "C" int32_t zkb_transcript_script_host(int32_t kind, const uint8_t *ops, uint64_t n_ops, const uint64_t *operands, uint8_t *proof, uint64_t cap,
                                               uint64_t *proof_len, uint64_t *challenges) {
-    ZKB_ARG(kind >= 0 && kind <= 2 && (ops || n_ops == 0) && proof_len);
-    zkb_session s;  // no pk, no device pool: only the transcript members are touched
-    s.tkind = kind;
+    ZKB_ARG(kind >= TR_BLAKE2B && kind <= TR_EVM && (ops || n_ops == 0) && proof_len);
+    Transcript t;
+    t.kind = (TranscriptKind)kind;
     const uint64_t *op = operands;
     for (uint64_t i = 0; i < n_ops; ++i) {
         switch (ops[i]) {
@@ -711,7 +720,7 @@ extern "C" int32_t zkb_transcript_script_host(int32_t kind, const uint8_t *ops, 
                 Fr v;
                 memcpy(v.l, op, 32);
                 op += 4;
-                if (ops[i] == 0) tr_common_scalar(&s, v); else tr_write_scalar(&s, v);
+                if (ops[i] == 0) t.common_scalar(v); else t.write_scalar(v);
                 break;
             }
             case 2: {
@@ -719,12 +728,12 @@ extern "C" int32_t zkb_transcript_script_host(int32_t kind, const uint8_t *ops, 
                 G1Affine p;
                 memcpy(&p, op, 64);
                 op += 8;
-                ZKB_TRY(tr_write_point(&s, p));
+                ZKB_TRY(t.write_point(p));
                 break;
             }
             case 3: {
                 ZKB_ARG(challenges);
-                const Fr c = tr_squeeze(&s);
+                const Fr c = t.squeeze();
                 memcpy(challenges, c.l, 32);
                 challenges += 4;
                 break;
@@ -732,10 +741,10 @@ extern "C" int32_t zkb_transcript_script_host(int32_t kind, const uint8_t *ops, 
             default: ZKB_ARG(false);
         }
     }
-    *proof_len = s.proof.size();
+    *proof_len = t.proof.size();
     if (proof) {
-        ZKB_ARG(cap >= s.proof.size());
-        if (!s.proof.empty()) memcpy(proof, s.proof.data(), s.proof.size());
+        ZKB_ARG(cap >= t.proof.size());
+        if (!t.proof.empty()) memcpy(proof, t.proof.data(), t.proof.size());
     }
     return ZKB_OK;
 }
@@ -749,15 +758,7 @@ extern "C" int32_t zkb_blake2b_challenge_host(const uint8_t *bytes, uint64_t len
     ZKB_ARG(out && (bytes || len == 0));
     Blake2b st("Halo2-Transcript");
     if (len) st.update(bytes, len);
-    const uint8_t pre = 0;
-    st.update(&pre, 1);
-    uint8_t h[64];
-    st.finalize_copy(h);
-    Fr lo, hi;
-    memcpy(lo.l, h, 32);
-    memcpy(hi.l, h + 32, 32);
-    const Fr r2 = Fr::r2();
-    const Fr c = fp_add(fp_mul(lo, r2), fp_mul(fp_mul(hi, r2), r2));
+    const Fr c = blake2b_challenge(st);
     memcpy(out, c.l, 32);
     return ZKB_OK;
 }
@@ -778,7 +779,7 @@ extern "C" int32_t zkb_pk_vk_bytes(zkb_pk *pk, uint8_t *out, uint64_t cap, uint6
     for (auto c : pk->fixed_values) cols.push_back(c);
     for (auto c : pk->sigma_values) cols.push_back(c);
     std::vector<G1Affine> cms;
-    if (!cols.empty()) ZKB_TRY(commit_many(pk, cols, pk->g_lagrange, pk->n, cms, st));
+    if (!cols.empty()) ZKB_TRY(commit_many(pk, BASIS_LAGRANGE, cols, cms, st));
     auto be32 = [](uint8_t *p, uint32_t v) { p[0] = (uint8_t)(v >> 24); p[1] = (uint8_t)(v >> 16); p[2] = (uint8_t)(v >> 8); p[3] = (uint8_t)v; };
     be32(out, cs.k);
     be32(out + 4, cs.nf);
@@ -859,13 +860,13 @@ static int32_t prove_begin_common(zkb_pk *pk, int32_t transcript_kind, const zkb
                                   const uint64_t *const *instance_values, const uint32_t *instance_lens, zkb_session **out);
 extern "C" int32_t zkb_prove_begin_ex(zkb_pk *pk, int32_t transcript_kind, const uint64_t transcript_repr[4], const uint64_t *const *instance_values,
                                       const uint32_t *instance_lens, zkb_session **out) {
-    ZKB_ARG(transcript_kind >= 0 && transcript_kind <= 2);
+    ZKB_ARG(transcript_kind >= TR_BLAKE2B && transcript_kind <= TR_EVM);
     return prove_begin_common(pk, transcript_kind, nullptr, transcript_repr, instance_values, instance_lens, out);
 }
 extern "C" int32_t zkb_prove_begin_cb(zkb_pk *pk, const zkb_transcript_vtable *vt, const uint64_t transcript_repr[4],
                                       const uint64_t *const *instance_values, const uint32_t *instance_lens, zkb_session **out) {
     ZKB_ARG(vt && vt->common_scalar && vt->write_scalar && vt->write_point && vt->squeeze_challenge);
-    return prove_begin_common(pk, 3, vt, transcript_repr, instance_values, instance_lens, out);
+    return prove_begin_common(pk, TR_CALLER, vt, transcript_repr, instance_values, instance_lens, out);
 }
 static int32_t prove_begin_common(zkb_pk *pk, int32_t transcript_kind, const zkb_transcript_vtable *vt, const uint64_t transcript_repr[4],
                                   const uint64_t *const *instance_values, const uint32_t *instance_lens, zkb_session **out) {
@@ -873,15 +874,15 @@ static int32_t prove_begin_common(zkb_pk *pk, int32_t transcript_kind, const zkb
     ZKB_CUDA(cudaSetDevice(pk->ctx->device));
     std::unique_ptr<zkb_session> s(new zkb_session());
     s->pk = pk;
-    s->tkind = transcript_kind;
-    if (vt) s->vt = *vt;
+    s->tr.kind = (TranscriptKind)transcript_kind;
+    if (vt) s->tr.vt = *vt;
     s->pool.ctx = pk->ctx;
     const Csf &cs = pk->cs;
     const uint64_t n = pk->n;
     cudaStream_t st = pk->ctx->stream;
     Fr repr;
     memcpy(repr.l, transcript_repr, 32);
-    tr_common_scalar(s.get(), repr);  // vk.hash_into(transcript)
+    s->tr.common_scalar(repr);  // vk.hash_into(transcript)
     s->inst_values.resize(cs.ni);
     s->inst_polys.resize(cs.ni);
     for (uint32_t c = 0; c < cs.ni; ++c) {
@@ -892,7 +893,7 @@ static int32_t prove_begin_common(zkb_pk *pk, int32_t transcript_kind, const zkb
         for (uint32_t i = 0; i < instance_lens[c]; ++i) {  // KZG: QUERY_INSTANCE = false -> values are absorbed as scalars
             Fr v;
             memcpy(v.l, instance_values[c] + 4 * i, 32);
-            tr_common_scalar(s.get(), v);
+            s->tr.common_scalar(v);
         }
         if (instance_lens[c]) ZKB_CUDA(cudaMemcpyAsync(s->inst_values[c], instance_values[c], (size_t)instance_lens[c] * sizeof(Fr), cudaMemcpyHostToDevice, st));
         ZKB_TRY(lagrange_to_coeff(pk, s->inst_values[c], s->inst_polys[c], st));
@@ -900,7 +901,7 @@ static int32_t prove_begin_common(zkb_pk *pk, int32_t transcript_kind, const zkb
     s->adv_values.assign(cs.na, nullptr);
     s->challenges.assign(cs.nch, Fr::zero());
     ZKB_CUDA(cudaStreamSynchronize(st));
-    if (s->cb_error) { set_error("the caller's transcript callback failed (%d)", s->cb_error); return ZKB_ERR_STATE; }
+    ZKB_TRY(s->tr.status());
     *out = s.release();
     return ZKB_OK;
 }
@@ -967,21 +968,18 @@ extern "C" int32_t zkb_prove_advice_phase(zkb_session *s, uint32_t phase, const 
     for (size_t b = 0; b < nbatch; ++b) {
         ZKB_CUDA(cudaStreamWaitEvent(st, evs[b], 0));
         const size_t lo = dealt ? 0 : b * maxb, hi = dealt ? ncols : std::min(ncols, (b + 1) * (size_t)maxb);
-        std::vector<Fr *> part(phase_cols.begin() + lo, phase_cols.begin() + hi);
-        std::vector<G1Affine> cms;
-        ZKB_TRY(commit_many(pk, part, pk->g_lagrange, n, cms, st));   // dealt: the same contiguous blocks as the uploads (same unit count)
-        for (auto &cm : cms) ZKB_TRY(tr_write_point(s, cm));
+        const std::vector<Fr *> part(phase_cols.begin() + lo, phase_cols.begin() + hi);
+        ZKB_TRY(commit_write(s, BASIS_LAGRANGE, part, st));   // dealt: the same contiguous blocks as the uploads (same unit count)
     }
     ZKB_TRY(deal_gather(pk->ctx, deal, slab, n * sizeof(Fr), st));   // column data of the other ranks' blocks over NVLink
     for (uint32_t i = 0; i < cs.nch; ++i) {
         if (cs.ch_phase[i] == phase) {
-            s->challenges[i] = tr_squeeze(s);
+            s->challenges[i] = s->tr.squeeze();
             if (challenges_out) memcpy(challenges_out + 4 * i, s->challenges[i].l, 32);
         }
     }
     s->next_phase++;
-    if (s->cb_error) { set_error("the caller's transcript callback failed (%d)", s->cb_error); return ZKB_ERR_STATE; }
-    return ZKB_OK;
+    return s->tr.status();
 }
 
 extern "C" int32_t zkb_session_destroy(zkb_session *s) {
@@ -1026,47 +1024,86 @@ struct OpenQuery {
     Fr point;
     Fr eval;
 };
+// SHPLONK: a committed polynomial with the rotations it is opened at, and a set of polynomials opened at the same rotations
+struct ShplonkCommit { int id; const Fr *poly; std::vector<int64_t> rots; };
+struct RotationSet {
+    std::vector<int64_t> rots;
+    std::vector<const ShplonkCommit *> comms;
+    std::vector<Fr> pts;                       // x * omega^rot of every rotation
+    std::vector<std::vector<Fr>> r_coeffs;     // per commitment: low-degree interpolant through (pts, evaluations)
+};
 
-static int32_t prove_finish_impl(zkb_session *s, const uint64_t *z_blinds, const uint64_t *phi_blinds, const uint64_t *random_poly_host) {
-    zkb_pk *pk = s->pk;
-    zkb_ctx *ctx = pk->ctx;
-    const Csf &cs = pk->cs;
-    const uint64_t n = pk->n;
-    const uint32_t bf = cs.bf, k = cs.k;
-    const uint32_t usable = (uint32_t)(n - bf - 1);
-    cudaStream_t st = ctx->stream;
-    DevPool &pool = s->pool;
+// What the stages of one create_proof hand to each other; lives for one call of prove_finish_impl.
+struct ProofState {
+    zkb_session *s;
+    zkb_pk *pk;
+    zkb_ctx *ctx;
+    const Csf &cs;
+    uint64_t n;
+    uint32_t k, bf;
+    cudaStream_t st;
+    DevPool &pool;
+    Deal lk_deal;   // multi-GPU: the lookup arguments are dealt, prepared and summed by the rank that owns them
+    Fr theta, beta, gamma, y, x, sy, sv, su;   // sy, sv, su: SHPLONK's y, v, u
+    Fr **d_vcols = nullptr;   // value-domain column table: [fixed | advice | instance | sigma | omega_pows]
+    std::vector<std::vector<Fr *>> lk_f;      // compressed inputs per lookup / input set
+    std::vector<Fr *> lk_t, lk_m, zs, phis;   // compressed tables, multiplicities, permutation grand products, lookup grand sums
+    Fr *random_poly = nullptr;
+    std::vector<Fr *> adv_polys, z_polys, phi_polys, m_polys;   // coefficient forms
+    // quotient: coset-domain slot table [fixed | advice | instance | sigma | z | phi | m | l0 | l_last | l_blind | X]; the program
+    // (common body + one trailing STOREACC slot rewritten per coset part); h on the extended domain, then its d - 1 pieces
+    std::vector<Fr *> qpolys;
+    uint32_t q_sigma0 = 0, q_z0 = 0, q_phi0 = 0, q_m0 = 0, q_l0 = 0;
+    DeviceProgram qdp;
+    size_t q_base_len = 0;
+    std::vector<uint32_t> tinv_idx;
+    Fr *h_ext = nullptr;
+    // openings: queries in multiopen order, the point of every rotation, the evaluation of every (polynomial, rotation)
+    std::vector<OpenQuery> queries;
+    std::map<int64_t, Fr> point_of;
+    std::map<std::pair<int, int64_t>, Fr> eval_of;
+    // SHPLONK: commitments (the sets point into this vector), rotation sets, the union of their rotations, h_x, work buffers
+    std::vector<ShplonkCommit> sh_commits;
+    std::vector<RotationSet> rsets;
+    std::vector<int64_t> super_rots;
+    Fr *hx = nullptr, *work = nullptr, *work2 = nullptr, *d_small = nullptr;
+
+    explicit ProofState(zkb_session *sess)
+        : s(sess), pk(sess->pk), ctx(pk->ctx), cs(pk->cs), n(pk->n), k(pk->cs.k), bf(pk->cs.bf), st(pk->ctx->stream), pool(sess->pool),
+          lk_deal(pk->ctx, pk->cs.lookups.size()) {}
+};
+
+// mv_lookup/prover.rs::prepare: compress inputs and table with theta, multiplicities m over the usable rows, commit m
+static int32_t lookups_prepare(ProofState &p) {
+    zkb_session *s = p.s;
+    const Csf &cs = p.cs;
+    const uint64_t n = p.n;
+    const uint32_t usable = (uint32_t)(n - p.bf - 1);
     const size_t nl = cs.lookups.size();
-    const Fr one = Fr::one();
-
-    // ---------------------------------------------------------------- theta; mv-lookup prepare (compress, multiplicities)
-    StageTrace trace(st);
-    const Fr theta = tr_squeeze(s);
-    // value-domain column table: [fixed | advice | instance | sigma | omega_pows]
+    cudaStream_t st = p.st;
+    DevPool &pool = p.pool;
     const SlotMap vsm{0, cs.nf, cs.nf + cs.na};
-    const uint32_t v_sigma0 = cs.nf + cs.na + cs.ni, v_omega = v_sigma0 + (uint32_t)cs.perm.size();
     std::vector<Fr *> vcols;
-    for (auto p : pk->fixed_values) vcols.push_back(p);
-    for (auto p : s->adv_values) vcols.push_back(p);
-    for (auto p : s->inst_values) vcols.push_back(p);
-    for (auto p : pk->sigma_values) vcols.push_back(p);
-    vcols.push_back(pk->omega_pows);
-    Fr **d_vcols = nullptr;
-    ZKB_TRY(upload_table(pool, vcols, &d_vcols, st));
+    for (auto q : p.pk->fixed_values) vcols.push_back(q);
+    for (auto q : s->adv_values) vcols.push_back(q);
+    for (auto q : s->inst_values) vcols.push_back(q);
+    for (auto q : p.pk->sigma_values) vcols.push_back(q);
+    vcols.push_back(p.pk->omega_pows);
+    ZKB_TRY(upload_table(pool, vcols, &p.d_vcols, st));
 
-    std::vector<std::vector<Fr *>> lk_f(nl);   // compressed inputs per lookup / input set
-    std::vector<Fr *> lk_t(nl), lk_m(nl);
-    // multi-GPU: lookup argument l is prepared by rank l mod P; m columns live in one slab (+ one word carrying error counts)
-    const Deal lk_deal(ctx, nl);
-    const bool lk_dealt = lk_deal.on;
+    p.lk_f.resize(nl);
+    p.lk_t.resize(nl);
+    p.lk_m.resize(nl);
+    // m columns live in one slab, completed by one all-gather when dealt
+    const Deal &deal = p.lk_deal;
     Fr *m_slab = nullptr;
     if (nl) {
-        ZKB_TRY(pool.fr(lk_deal.padded() * n, &m_slab));
-        for (size_t l = 0; l < nl; ++l) lk_m[l] = m_slab + l * n;
+        ZKB_TRY(pool.fr(deal.padded() * n, &m_slab));
+        for (size_t l = 0; l < nl; ++l) p.lk_m[l] = m_slab + l * n;
     }
     uint64_t lookup_errors = 0;
     for (size_t l = 0; l < nl; ++l) {
-        if (!lk_deal.mine(l)) continue;
+        if (!deal.mine(l)) continue;
         const CsfLookup &lk = cs.lookups[l];
         ExprBuilder eb;
         ProgramBuilder pb(eb);
@@ -1076,19 +1113,15 @@ static int32_t prove_finish_impl(zkb_session *s, const uint64_t *z_blinds, const
         for (size_t j = 0; j < lk.inputs.size(); ++j) {
             Fr *a;
             ZKB_TRY(pool.fr(n, &a));
-            lk_f[l].push_back(a);
+            p.lk_f[l].push_back(a);
             outs.push_back(a);
-            roots.push_back({compress_exprs(cs, lk.inputs[j], eb, vsm, s->challenges, memo, theta), ProgramBuilder::STORE, (uint32_t)j});
+            roots.push_back({compress_exprs(cs, lk.inputs[j], eb, vsm, s->challenges, memo, p.theta), ProgramBuilder::STORE, (uint32_t)j});
         }
-        ZKB_TRY(pool.fr(n, &lk_t[l]));
-        outs.push_back(lk_t[l]);
-        roots.push_back({compress_exprs(cs, lk.table, eb, vsm, s->challenges, memo, theta), ProgramBuilder::STORE, (uint32_t)lk.inputs.size()});
+        ZKB_TRY(pool.fr(n, &p.lk_t[l]));
+        outs.push_back(p.lk_t[l]);
+        roots.push_back({compress_exprs(cs, lk.table, eb, vsm, s->challenges, memo, p.theta), ProgramBuilder::STORE, (uint32_t)lk.inputs.size()});
         if (!pb.scope(roots)) { set_error("lookup %zu: %s", l, pb.error.c_str()); return ZKB_ERR_ARG; }
-        DeviceProgram dp;
-        ZKB_TRY(upload_program(pool, pb, eb, dp, st));
-        Fr **d_outs = nullptr;
-        ZKB_TRY(upload_table(pool, outs, &d_outs, st));
-        ZKB_TRY(expr_run_device(ctx, dp.code, dp.ncode, dp.nregs, d_vcols, dp.consts, d_outs, k, 1, 0, st));
+        ZKB_TRY(run_program(s, pb, eb, p.d_vcols, outs, st));
         // multiplicities over the usable rows
         uint32_t tsize = 1;
         while (tsize < 2 * usable) tsize <<= 1;
@@ -1100,25 +1133,25 @@ static int32_t prove_finish_impl(zkb_session *s, const uint64_t *z_blinds, const
         ZKB_CUDA(cudaMemsetAsync(slots, 0, (size_t)tsize * 4, st));
         ZKB_CUDA(cudaMemsetAsync(counts, 0, (size_t)n * 4 + 16, st));
         const unsigned ub = (usable + 255) / 256;
-        m_insert_kernel<<<ub, 256, 0, st>>>(lk_t[l], usable, slots, tsize - 1);
-        for (size_t j = 0; j < lk.inputs.size(); ++j) m_count_kernel<<<ub, 256, 0, st>>>(lk_f[l][j], lk_t[l], usable, slots, tsize - 1, counts, d_err);
-        counts_to_fr_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(counts, (uint32_t)n, lk_m[l]);
-        ctx->launches += 2 + lk.inputs.size();
+        m_insert_kernel<<<ub, 256, 0, st>>>(p.lk_t[l], usable, slots, tsize - 1);
+        for (size_t j = 0; j < lk.inputs.size(); ++j) m_count_kernel<<<ub, 256, 0, st>>>(p.lk_f[l][j], p.lk_t[l], usable, slots, tsize - 1, counts, d_err);
+        counts_to_fr_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(counts, (uint32_t)n, p.lk_m[l]);
+        p.ctx->launches += 2 + lk.inputs.size();
         int herr = 0;
         ZKB_CUDA(cudaMemcpyAsync(&herr, d_err, 4, cudaMemcpyDeviceToHost, st));
         ZKB_CUDA(cudaStreamSynchronize(st));
         if (herr) {
             set_error("lookup %zu: an input row is not in the table (unsatisfied witness)", l);
-            if (!lk_dealt) return ZKB_ERR_ARG;
+            if (!deal.on) return ZKB_ERR_ARG;
             lookup_errors++;   // multi-GPU: every rank must learn about it before anyone leaves the collective sequence
         }
     }
-    if (lk_dealt) {
-        ZKB_TRY(deal_gather(ctx, lk_deal, m_slab, n * sizeof(Fr), st));
+    if (deal.on) {
+        ZKB_TRY(deal_gather(p.ctx, deal, m_slab, n * sizeof(Fr), st));
         uint64_t *d_errw = nullptr;   // every rank learns about an unsatisfied lookup before anyone leaves the collective sequence
-        ZKB_TRY(scratch_get(ctx, SCR_COMM_FLAG, 64, (void **)&d_errw));
+        ZKB_TRY(scratch_get(p.ctx, SCR_COMM_FLAG, 64, (void **)&d_errw));
         ZKB_CUDA(cudaMemcpyAsync(d_errw + 1, &lookup_errors, 8, cudaMemcpyHostToDevice, st));
-        ZKB_TRY(comm_allreduce_u64(ctx, d_errw + 1, 1, st));
+        ZKB_TRY(comm_allreduce_u64(p.ctx, d_errw + 1, 1, st));
         uint64_t total_err = 0;
         ZKB_CUDA(cudaMemcpyAsync(&total_err, d_errw + 1, 8, cudaMemcpyDeviceToHost, st));
         ZKB_CUDA(cudaStreamSynchronize(st));
@@ -1127,117 +1160,102 @@ static int32_t prove_finish_impl(zkb_session *s, const uint64_t *z_blinds, const
             return ZKB_ERR_ARG;
         }
     }
-    {
-        std::vector<G1Affine> cms;
-        ZKB_TRY(commit_many(pk, lk_m, pk->g_lagrange, n, cms, st));
-        for (auto &cm : cms) ZKB_TRY(tr_write_point(s, cm));
-    }
+    return commit_write(s, BASIS_LAGRANGE, p.lk_m, st);
+}
 
-    trace.mark("lookups: compress + m + commit");
-    // ---------------------------------------------------------------- beta, gamma; permutation grand products
-    const Fr beta = tr_squeeze(s);
-    const Fr gamma = tr_squeeze(s);
-    auto perm_slot_values = [&](const std::array<uint32_t, 2> &c) -> uint32_t {
-        return c[0] == N_FIXED ? vsm.fixed0 + c[1] : c[0] == N_ADVICE ? vsm.advice0 + c[1] : vsm.instance0 + c[1];
-    };
-    std::vector<Fr *> zs(pk->nsets);
-    {
-        Fr delta;
-        {   // DELTA = 7^(2^28)
-            Fr seven = fr_from_u64(7);
-            delta = seven;
-            for (int i = 0; i < 28; ++i) delta = fp_sqr(delta);
+// permutation/prover.rs: grand products z of the permutation sets (z_blinds: bf values per set), commit z
+static int32_t permutation_commit(ProofState &p, const uint64_t *z_blinds) {
+    zkb_pk *pk = p.pk;
+    zkb_ctx *ctx = p.ctx;
+    const Csf &cs = p.cs;
+    const uint64_t n = p.n;
+    const uint32_t bf = p.bf;
+    cudaStream_t st = p.st;
+    const Fr one = Fr::one();
+    const SlotMap vsm{0, cs.nf, cs.nf + cs.na};
+    const uint32_t v_sigma0 = cs.nf + cs.na + cs.ni, v_omega = v_sigma0 + (uint32_t)cs.perm.size();
+    const Fr delta = perm_delta();
+    // Multi-GPU: the sets are dealt.  Upstream chains them (z_i[0] = last value of z_{i-1}), which is sequential; here every set is
+    // scanned from 1 and rescaled afterwards by c_i = product of the previous sets' last values -- the same field elements
+    // (z_i = c_i * z'_i row by row), with only the nsets last values crossing the ranks before the columns are gathered.
+    const Deal dp_sets(ctx, pk->nsets);
+    p.zs.resize(pk->nsets);
+    Fr *z_slab = nullptr;
+    ZKB_TRY(p.pool.fr(std::max<size_t>(1, dp_sets.padded()) * n, &z_slab));
+    for (uint32_t si = 0; si < pk->nsets; ++si) p.zs[si] = z_slab + (size_t)si * n;
+    Fr *num, *den, *tmp;
+    ZKB_TRY(p.pool.fr(n, &num));
+    ZKB_TRY(p.pool.fr(n, &den));
+    ZKB_TRY(p.pool.fr(n, &tmp));
+    std::vector<Fr> lasts(std::max<size_t>(1, dp_sets.padded()), one);
+    Fr last_z = one;
+    for (uint32_t si = 0; si < pk->nsets; ++si) {
+        if (!dp_sets.mine(si)) continue;
+        ExprBuilder eb;
+        ProgramBuilder pb(eb);
+        uint32_t nnum = 0, nden = 0;
+        bool first = true;
+        Fr delta_pow = fp_pow_u64(delta, (uint64_t)si * pk->chunk);
+        for (uint32_t j = si * pk->chunk; j < std::min<size_t>((si + 1) * pk->chunk, cs.perm.size()); ++j) {
+            const uint32_t v = eb.col(perm_slot(vsm, cs.perm[j]), 0);
+            const uint32_t dterm = eb.add(eb.add(v, eb.mul(eb.col(v_sigma0 + j, 0), eb.constant(p.beta))), eb.constant(p.gamma));
+            const uint32_t nterm = eb.add(eb.add(v, eb.mul(eb.col(v_omega, 0), eb.constant(fp_mul(p.beta, delta_pow)))), eb.constant(p.gamma));
+            nden = first ? dterm : eb.mul(nden, dterm);
+            nnum = first ? nterm : eb.mul(nnum, nterm);
+            first = false;
+            delta_pow = fp_mul(delta_pow, delta);
         }
-        // Multi-GPU: the sets are dealt.  Upstream chains them (z_i[0] = last value of z_{i-1}), which is sequential; here every set is
-        // scanned from 1 and rescaled afterwards by c_i = product of the previous sets' last values -- the same field elements
-        // (z_i = c_i * z'_i row by row), with only the nsets last values crossing the ranks before the columns are gathered.
-        const Deal dp_sets(ctx, pk->nsets);
-        Fr *z_slab = nullptr;
-        ZKB_TRY(pool.fr(std::max<size_t>(1, dp_sets.padded()) * n, &z_slab));
-        for (uint32_t si = 0; si < pk->nsets; ++si) zs[si] = z_slab + (size_t)si * n;
-        Fr *num, *den, *tmp;
-        ZKB_TRY(pool.fr(n, &num));
-        ZKB_TRY(pool.fr(n, &den));
-        ZKB_TRY(pool.fr(n, &tmp));
-        std::vector<Fr> lasts(std::max<size_t>(1, dp_sets.padded()), one);
-        Fr last_z = one;
+        if (!pb.scope({{nnum, ProgramBuilder::STORE, 0}, {nden, ProgramBuilder::STORE, 1}})) { set_error("permutation: %s", pb.error.c_str()); return ZKB_ERR_ARG; }
+        ZKB_TRY(run_program(p.s, pb, eb, p.d_vcols, {num, den}, st));
+        ZKB_TRY(batch_invert_device(ctx, den, tmp, n, st));
+        mul_arrays_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(num, tmp, den, n);  // den <- modified values
+        ctx->launches++;
+        // one GPU: chained exactly like upstream (init = previous last value); dealt: from 1, rescaled below
+        ZKB_TRY(prefix_product_device(ctx, den, n, dp_sets.on ? one : last_z, p.zs[si], st));
+        ZKB_CUDA(cudaMemcpyAsync(&last_z, p.zs[si] + (n - bf - 1), sizeof(Fr), cudaMemcpyDeviceToHost, st));
+        ZKB_CUDA(cudaStreamSynchronize(st));
+        lasts[si] = last_z;
+        if (!dp_sets.on) ZKB_CUDA(cudaMemcpyAsync(p.zs[si] + (n - bf), z_blinds + 4ull * bf * si, (size_t)bf * sizeof(Fr), cudaMemcpyHostToDevice, st));
+    }
+    if (dp_sets.on) {
+        ZKB_TRY(deal_gather_host(ctx, dp_sets, lasts.data(), sizeof(Fr), st));
+        Fr c = one;   // c_i = prod_{j < i} last'_j
         for (uint32_t si = 0; si < pk->nsets; ++si) {
-            if (!dp_sets.mine(si)) continue;
-            ExprBuilder eb;
-            ProgramBuilder pb(eb);
-            uint32_t nnum = 0, nden = 0;
-            bool first = true;
-            Fr delta_pow = fp_pow_u64(delta, (uint64_t)si * pk->chunk);
-            for (uint32_t j = si * pk->chunk; j < std::min<size_t>((si + 1) * pk->chunk, cs.perm.size()); ++j) {
-                const uint32_t v = eb.col(perm_slot_values(cs.perm[j]), 0);
-                const uint32_t dterm = eb.add(eb.add(v, eb.mul(eb.col(v_sigma0 + j, 0), eb.constant(beta))), eb.constant(gamma));
-                const uint32_t nterm = eb.add(eb.add(v, eb.mul(eb.col(v_omega, 0), eb.constant(fp_mul(beta, delta_pow)))), eb.constant(gamma));
-                nden = first ? dterm : eb.mul(nden, dterm);
-                nnum = first ? nterm : eb.mul(nnum, nterm);
-                first = false;
-                delta_pow = fp_mul(delta_pow, delta);
+            if (dp_sets.mine(si)) {
+                if (!(c == one)) { scale_const_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(p.zs[si], c, n); ctx->launches++; }
+                ZKB_CUDA(cudaMemcpyAsync(p.zs[si] + (n - bf), z_blinds + 4ull * bf * si, (size_t)bf * sizeof(Fr), cudaMemcpyHostToDevice, st));
             }
-            if (!pb.scope({{nnum, ProgramBuilder::STORE, 0}, {nden, ProgramBuilder::STORE, 1}})) { set_error("permutation: %s", pb.error.c_str()); return ZKB_ERR_ARG; }
-            DeviceProgram dp;
-            ZKB_TRY(upload_program(pool, pb, eb, dp, st));
-            std::vector<Fr *> outs{num, den};
-            Fr **d_outs = nullptr;
-            ZKB_TRY(upload_table(pool, outs, &d_outs, st));
-            ZKB_TRY(expr_run_device(ctx, dp.code, dp.ncode, dp.nregs, d_vcols, dp.consts, d_outs, k, 1, 0, st));
-            ZKB_TRY(batch_invert_device(ctx, den, tmp, n, st));
-            mul_arrays_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(num, tmp, den, n);  // den <- modified values
-            ctx->launches++;
-            // one GPU: chained exactly like upstream (init = previous last value); dealt: from 1, rescaled below
-            ZKB_TRY(prefix_product_device(ctx, den, n, dp_sets.on ? one : last_z, zs[si], st));
-            ZKB_CUDA(cudaMemcpyAsync(&last_z, zs[si] + (n - bf - 1), sizeof(Fr), cudaMemcpyDeviceToHost, st));
-            ZKB_CUDA(cudaStreamSynchronize(st));
-            lasts[si] = last_z;
-            if (!dp_sets.on) ZKB_CUDA(cudaMemcpyAsync(zs[si] + (n - bf), z_blinds + 4ull * bf * si, (size_t)bf * sizeof(Fr), cudaMemcpyHostToDevice, st));
+            c = fp_mul(c, lasts[si]);
         }
-        if (dp_sets.on) {
-            Fr *d_l = nullptr;
-            ZKB_TRY(scratch_get(ctx, SCR_COMM, dp_sets.padded() * sizeof(Fr), (void **)&d_l));
-            ZKB_CUDA(cudaMemcpyAsync(d_l, lasts.data(), dp_sets.padded() * sizeof(Fr), cudaMemcpyHostToDevice, st));
-            ZKB_TRY(deal_gather(ctx, dp_sets, d_l, sizeof(Fr), st));
-            ZKB_CUDA(cudaMemcpyAsync(lasts.data(), d_l, dp_sets.padded() * sizeof(Fr), cudaMemcpyDeviceToHost, st));
-            ZKB_CUDA(cudaStreamSynchronize(st));
-            Fr c = one;   // c_i = prod_{j < i} last'_j
-            for (uint32_t si = 0; si < pk->nsets; ++si) {
-                if (dp_sets.mine(si)) {
-                    if (!(c == one)) { scale_const_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(zs[si], c, n); ctx->launches++; }
-                    ZKB_CUDA(cudaMemcpyAsync(zs[si] + (n - bf), z_blinds + 4ull * bf * si, (size_t)bf * sizeof(Fr), cudaMemcpyHostToDevice, st));
-                }
-                c = fp_mul(c, lasts[si]);
-            }
-            ZKB_TRY(deal_gather(ctx, dp_sets, z_slab, n * sizeof(Fr), st));
-        }
+        ZKB_TRY(deal_gather(ctx, dp_sets, z_slab, n * sizeof(Fr), st));
     }
-    {
-        std::vector<G1Affine> cms;
-        ZKB_TRY(commit_many(pk, zs, pk->g_lagrange, n, cms, st));
-        for (auto &cm : cms) ZKB_TRY(tr_write_point(s, cm));
-    }
+    return commit_write(p.s, BASIS_LAGRANGE, p.zs, st);
+}
 
-    trace.mark("permutation z + commit");
-    // ---------------------------------------------------------------- lookup grand sums phi
-    std::vector<Fr *> phis(nl);
+// mv_lookup/prover.rs::commit_grand_sum: phi = prefix sum of sum_j 1/(f_j + beta) - m/(t + beta) (phi_blinds: bf values per lookup)
+static int32_t lookups_commit_sums(ProofState &p, const uint64_t *phi_blinds) {
+    const uint64_t n = p.n;
+    const size_t nl = p.cs.lookups.size();
+    cudaStream_t st = p.st;
+    DevPool &pool = p.pool;
+    p.phis.resize(nl);
     Fr *phi_slab = nullptr;
     if (nl) {
-        ZKB_TRY(pool.fr(lk_deal.padded() * n, &phi_slab));
-        for (size_t l = 0; l < nl; ++l) phis[l] = phi_slab + l * n;
+        ZKB_TRY(pool.fr(p.lk_deal.padded() * n, &phi_slab));
+        for (size_t l = 0; l < nl; ++l) p.phis[l] = phi_slab + l * n;
     }
     for (size_t l = 0; l < nl; ++l) {
-        if (!lk_deal.mine(l)) continue;
-        const size_t J = lk_f[l].size();
+        if (!p.lk_deal.mine(l)) continue;
+        const size_t J = p.lk_f[l].size();
         // denominators (f_j + beta), (t + beta) into one contiguous array, inverted at once
         Fr *dens, *invs, *dterm;
         ZKB_TRY(pool.fr((J + 1) * n, &dens));
         ZKB_TRY(pool.fr((J + 1) * n, &invs));
         ZKB_TRY(pool.fr(n, &dterm));
         std::vector<Fr *> cols;
-        for (auto p : lk_f[l]) cols.push_back(p);
-        cols.push_back(lk_t[l]);          // slot J
-        cols.push_back(lk_m[l]);          // slot J + 1
+        for (auto q : p.lk_f[l]) cols.push_back(q);
+        cols.push_back(p.lk_t[l]);          // slot J
+        cols.push_back(p.lk_m[l]);          // slot J + 1
         for (size_t j = 0; j <= J; ++j) cols.push_back(invs + j * n);  // slots J + 2 ..
         Fr **d_cols = nullptr;
         ZKB_TRY(upload_table(pool, cols, &d_cols, st));
@@ -1247,223 +1265,202 @@ static int32_t prove_finish_impl(zkb_session *s, const uint64_t *z_blinds, const
             std::vector<ProgramBuilder::Root> roots;
             std::vector<Fr *> outs;
             for (size_t j = 0; j <= J; ++j) {
-                roots.push_back({eb.add(eb.col((uint32_t)j, 0), eb.constant(beta)), ProgramBuilder::STORE, (uint32_t)j});
+                roots.push_back({eb.add(eb.col((uint32_t)j, 0), eb.constant(p.beta)), ProgramBuilder::STORE, (uint32_t)j});
                 outs.push_back(dens + j * n);
             }
             if (!pb.scope(roots)) { set_error("lookup sum: %s", pb.error.c_str()); return ZKB_ERR_ARG; }
-            DeviceProgram dp;
-            ZKB_TRY(upload_program(pool, pb, eb, dp, st));
-            Fr **d_outs = nullptr;
-            ZKB_TRY(upload_table(pool, outs, &d_outs, st));
-            ZKB_TRY(expr_run_device(ctx, dp.code, dp.ncode, dp.nregs, d_cols, dp.consts, d_outs, k, 1, 0, st));
+            ZKB_TRY(run_program(p.s, pb, eb, d_cols, outs, st));
         }
-        ZKB_TRY(batch_invert_device(ctx, dens, invs, (J + 1) * n, st));
+        ZKB_TRY(batch_invert_device(p.ctx, dens, invs, (J + 1) * n, st));
         {
             ExprBuilder eb;
             ProgramBuilder pb(eb);
             uint32_t acc = eb.neg(eb.mul(eb.col((uint32_t)J + 1, 0), eb.col((uint32_t)(J + 2 + J), 0)));  // - m / (t + beta)
             for (size_t j = 0; j < J; ++j) acc = eb.add(acc, eb.col((uint32_t)(J + 2 + j), 0));
             if (!pb.scope({{acc, ProgramBuilder::STORE, 0}})) { set_error("lookup sum: %s", pb.error.c_str()); return ZKB_ERR_ARG; }
-            DeviceProgram dp;
-            ZKB_TRY(upload_program(pool, pb, eb, dp, st));
-            std::vector<Fr *> outs{dterm};
-            Fr **d_outs = nullptr;
-            ZKB_TRY(upload_table(pool, outs, &d_outs, st));
-            ZKB_TRY(expr_run_device(ctx, dp.code, dp.ncode, dp.nregs, d_cols, dp.consts, d_outs, k, 1, 0, st));
+            ZKB_TRY(run_program(p.s, pb, eb, d_cols, {dterm}, st));
         }
-        ZKB_TRY(prefix_sum_device(ctx, dterm, n, Fr::zero(), phis[l], st));
-        ZKB_CUDA(cudaMemcpyAsync(phis[l] + (n - bf), phi_blinds + 4ull * bf * l, (size_t)bf * sizeof(Fr), cudaMemcpyHostToDevice, st));
+        ZKB_TRY(prefix_sum_device(p.ctx, dterm, n, Fr::zero(), p.phis[l], st));
+        ZKB_CUDA(cudaMemcpyAsync(p.phis[l] + (n - p.bf), phi_blinds + 4ull * p.bf * l, (size_t)p.bf * sizeof(Fr), cudaMemcpyHostToDevice, st));
     }
-    if (nl) ZKB_TRY(deal_gather(ctx, lk_deal, phi_slab, n * sizeof(Fr), st));
-    {
-        std::vector<G1Affine> cms;
-        ZKB_TRY(commit_many(pk, phis, pk->g_lagrange, n, cms, st));
-        for (auto &cm : cms) ZKB_TRY(tr_write_point(s, cm));
-    }
+    if (nl) ZKB_TRY(deal_gather(p.ctx, p.lk_deal, phi_slab, n * sizeof(Fr), st));
+    return commit_write(p.s, BASIS_LAGRANGE, p.phis, st);
+}
 
-    trace.mark("lookup phi + commit");
-    // ---------------------------------------------------------------- vanishing: random polynomial
-    Fr *random_poly;
-    ZKB_TRY(pool.fr(n, &random_poly));
-    ZKB_CUDA(cudaMemcpyAsync(random_poly, random_poly_host, n * sizeof(Fr), cudaMemcpyHostToDevice, st));
-    {
-        G1Affine cm;
-        { std::vector<Fr *> one_col{random_poly}; std::vector<G1Affine> r1; ZKB_TRY(commit_many(pk, one_col, pk->g, n, r1, st)); cm = r1[0]; }
-        ZKB_TRY(tr_write_point(s, cm));
-    }
-    const Fr y = tr_squeeze(s);
+// vanishing/prover.rs commit: the caller's random polynomial (n coefficients), committed with g
+static int32_t vanishing_commit_random(ProofState &p, const uint64_t *random_poly_host) {
+    ZKB_TRY(p.pool.fr(p.n, &p.random_poly));
+    ZKB_CUDA(cudaMemcpyAsync(p.random_poly, random_poly_host, p.n * sizeof(Fr), cudaMemcpyHostToDevice, p.st));
+    return commit_write(p.s, BASIS_G, {p.random_poly}, p.st);
+}
 
-    trace.mark("random poly commit");
-    // ---------------------------------------------------------------- coefficient forms
-    const uint32_t ntt_chunk = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(256, (1ull << 31) / (n * sizeof(Fr))));  // <= 2 GiB of NTT scratch
-    auto ntt_many = [&](const std::vector<Fr *> &src, const std::vector<Fr *> &dst, const Fr &w, const Fr *scale, const Fr *in_scale) -> int32_t {
-        for (size_t done = 0; done < src.size(); done += ntt_chunk) {
-            const uint32_t cur = (uint32_t)std::min<size_t>(ntt_chunk, src.size() - done);
-            std::vector<Fr *> a(src.begin() + done, src.begin() + done + cur), b(dst.begin() + done, dst.begin() + done + cur);
-            ZKB_TRY(ntt_fr_batch_device(ctx, a.data(), b.data(), cur, k, w, scale, 0, in_scale, st));
-        }
-        return ZKB_OK;
+// size-n transforms of src[i] into dst[i], batched with at most 2 GiB of NTT scratch per launch
+static int32_t ntt_many(ProofState &p, const std::vector<Fr *> &src, const std::vector<Fr *> &dst, const Fr &w, const Fr *scale, const Fr *in_scale) {
+    const uint32_t chunk = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(256, (1ull << 31) / (p.n * sizeof(Fr))));
+    for (size_t done = 0; done < src.size(); done += chunk) {
+        const uint32_t cur = (uint32_t)std::min<size_t>(chunk, src.size() - done);
+        std::vector<Fr *> a(src.begin() + done, src.begin() + done + cur), b(dst.begin() + done, dst.begin() + done + cur);
+        ZKB_TRY(ntt_fr_batch_device(p.ctx, a.data(), b.data(), cur, p.k, w, scale, 0, in_scale, p.st));
+    }
+    return ZKB_OK;
+}
+// coefficient forms of `vals` in a new slab; multi-GPU: contiguous blocks of columns per rank, completed by one all-gather
+static int32_t to_coeff_new(ProofState &p, const std::vector<Fr *> &vals, std::vector<Fr *> &polys) {
+    polys.resize(vals.size());
+    if (vals.empty()) return ZKB_OK;
+    Fr *pslab = nullptr;
+    const Deal dc(p.ctx, vals.size());
+    ZKB_TRY(p.pool.fr(dc.padded() * p.n, &pslab));
+    for (size_t i = 0; i < vals.size(); ++i) polys[i] = pslab + i * p.n;
+    std::vector<Fr *> src, dst;
+    for (size_t i = 0; i < vals.size(); ++i)
+        if (dc.mine(i)) { src.push_back(vals[i]); dst.push_back(polys[i]); }
+    if (!src.empty()) ZKB_TRY(ntt_many(p, src, dst, p.pk->omega_inv, &p.pk->n_inv, nullptr));
+    return deal_gather(p.ctx, dc, pslab, p.n * sizeof(Fr), p.st);
+}
+static int32_t to_coefficients(ProofState &p) {
+    ZKB_TRY(to_coeff_new(p, p.s->adv_values, p.adv_polys));
+    ZKB_TRY(to_coeff_new(p, p.zs, p.z_polys));
+    ZKB_TRY(to_coeff_new(p, p.phis, p.phi_polys));
+    return to_coeff_new(p, p.lk_m, p.m_polys);
+}
+
+// evaluation.rs::evaluate_h: the quotient numerator as ONE interpreter program over the coset-domain slot table, every constraint
+// folded in with Horner in y, in upstream's order (gates, permutation, lookups)
+static int32_t quotient_program(ProofState &p) {
+    zkb_pk *pk = p.pk;
+    const Csf &cs = p.cs;
+    const std::vector<Fr> &challenges = p.s->challenges;
+    const Fr one = Fr::one();
+    auto append = [&](const std::vector<Fr *> &polys) {   // -> first slot of `polys`
+        const uint32_t at = (uint32_t)p.qpolys.size();
+        p.qpolys.insert(p.qpolys.end(), polys.begin(), polys.end());
+        return at;
     };
-    auto to_coeff_new = [&](const std::vector<Fr *> &vals, std::vector<Fr *> &polys) -> int32_t {
-        polys.resize(vals.size());
-        if (vals.empty()) return ZKB_OK;
-        Fr *pslab = nullptr;
-        const Deal dc(ctx, vals.size());   // multi-GPU: contiguous blocks of columns per rank, completed by one all-gather
-        ZKB_TRY(pool.fr(dc.padded() * n, &pslab));
-        for (size_t i = 0; i < vals.size(); ++i) polys[i] = pslab + i * n;
-        std::vector<Fr *> src, dst;
-        for (size_t i = 0; i < vals.size(); ++i)
-            if (dc.mine(i)) { src.push_back(vals[i]); dst.push_back(polys[i]); }
-        if (!src.empty()) ZKB_TRY(ntt_many(src, dst, pk->omega_inv, &pk->n_inv, nullptr));
-        ZKB_TRY(deal_gather(ctx, dc, pslab, n * sizeof(Fr), st));
-        return ZKB_OK;
-    };
-    std::vector<Fr *> adv_polys, z_polys, phi_polys, m_polys;
-    ZKB_TRY(to_coeff_new(s->adv_values, adv_polys));
-    ZKB_TRY(to_coeff_new(zs, z_polys));
-    ZKB_TRY(to_coeff_new(phis, phi_polys));
-    ZKB_TRY(to_coeff_new(lk_m, m_polys));
-
-    trace.mark("lagrange_to_coeff (all columns)");
-    // ---------------------------------------------------------------- quotient numerator program (plonk/evaluation.rs order)
-    // coset-domain slot table: [fixed | advice | instance | sigma | z | phi | m | l0 | l_last | l_blind | X]
-    std::vector<Fr *> qpolys;
-    for (auto p : pk->fixed_polys) qpolys.push_back(p);
-    for (auto p : adv_polys) qpolys.push_back(p);
-    for (auto p : s->inst_polys) qpolys.push_back(p);
-    const uint32_t q_sigma0 = (uint32_t)qpolys.size();
-    for (auto p : pk->sigma_polys) qpolys.push_back(p);
-    const uint32_t q_z0 = (uint32_t)qpolys.size();
-    for (auto p : z_polys) qpolys.push_back(p);
-    const uint32_t q_phi0 = (uint32_t)qpolys.size();
-    for (auto p : phi_polys) qpolys.push_back(p);
-    const uint32_t q_m0 = (uint32_t)qpolys.size();
-    for (auto p : m_polys) qpolys.push_back(p);
-    const uint32_t q_l0 = (uint32_t)qpolys.size();
-    qpolys.push_back(pk->l0_poly);
-    qpolys.push_back(pk->llast_poly);
-    qpolys.push_back(pk->lblind_poly);
-    qpolys.push_back(pk->xid_poly);
-    const uint32_t q_llast = q_l0 + 1, q_lblind = q_l0 + 2, q_x = q_l0 + 3;
-    ZKB_ARG(qpolys.size() < 65536);
+    append(pk->fixed_polys);
+    append(p.adv_polys);
+    append(p.s->inst_polys);
+    p.q_sigma0 = append(pk->sigma_polys);
+    p.q_z0 = append(p.z_polys);
+    p.q_phi0 = append(p.phi_polys);
+    p.q_m0 = append(p.m_polys);
+    p.q_l0 = append({pk->l0_poly, pk->llast_poly, pk->lblind_poly, pk->xid_poly});
+    const uint32_t q_l0 = p.q_l0, q_llast = q_l0 + 1, q_lblind = q_l0 + 2, q_x = q_l0 + 3;
+    ZKB_ARG(p.qpolys.size() < 65536);
     const SlotMap qsm{0, cs.nf, cs.nf + cs.na};
 
     ExprBuilder qeb;
     ProgramBuilder qpb(qeb);
-    const uint32_t y_idx = qeb.const_slot(y);
-    {
-        std::vector<int64_t> memo(cs.nodes.size(), -1);
-        // Gate polynomials, Horner in y in constraint-system order.  Circuits multiply whole groups of constraints by one selector
-        // (`q_enable * constraint`), so runs of CONSECUTIVE gates of the form fixed(col, rot) * t_j are folded exactly:
-        //   (..(acc y + f t_1) y + ..) y + f t_r  =  acc y^r + f (t_1 y^(r-1) + .. + t_r)
-        // -- the same field element (distributivity is exact mod r), one multiply per gate less than the term-by-term form.
-        auto selector_split = [&](uint32_t gnode, uint32_t &sel, uint32_t &rest) -> bool {
-            const auto &nd = cs.nodes[gnode];
-            if (nd[0] != N_MUL) return false;
-            for (int side = 0; side < 2; ++side) {
-                const uint32_t a = nd[1 + side], b = nd[2 - side];
-                if (cs.nodes[a][0] == N_FIXED) { sel = a; rest = b; return true; }
-            }
-            return false;
-        };
-        auto same_query = [&](uint32_t a, uint32_t b) { return cs.nodes[a][1] == cs.nodes[b][1] && cs.nodes[a][2] == cs.nodes[b][2]; };
-        const bool fold_runs = !(getenv("ZKB_NO_SELECTOR_FOLD") && getenv("ZKB_NO_SELECTOR_FOLD")[0] == '1');
-        for (size_t gi = 0; gi < cs.gates.size();) {
-            uint32_t sel = 0, rest = 0;
-            size_t run = 1;
-            if (fold_runs && selector_split(cs.gates[gi], sel, rest)) {
-                uint32_t s2 = 0, r2 = 0;
-                while (gi + run < cs.gates.size() && run < 4096 && selector_split(cs.gates[gi + run], s2, r2) && same_query(sel, s2)) ++run;
-            }
-            if (run < 2) {
-                if (!qpb.scope({{translate(cs, cs.gates[gi], qeb, qsm, s->challenges, memo), ProgramBuilder::HORNER, y_idx}})) { set_error("gate: %s", qpb.error.c_str()); return ZKB_ERR_ARG; }
-                ++gi;
-                continue;
-            }
-            for (size_t t = 0; t < run; ++t) {
-                uint32_t s2 = 0, r2 = 0;
-                selector_split(cs.gates[gi + t], s2, r2);
-                if (!qpb.scope({{translate(cs, r2, qeb, qsm, s->challenges, memo), ProgramBuilder::HORNER2, y_idx}})) { set_error("gate: %s", qpb.error.c_str()); return ZKB_ERR_ARG; }
-            }
-            const uint32_t yr_idx = qeb.const_slot(fp_pow_u64(y, run));
-            if (!qpb.scope({{translate(cs, sel, qeb, qsm, s->challenges, memo), ProgramBuilder::FOLD, yr_idx}})) { set_error("gate: %s", qpb.error.c_str()); return ZKB_ERR_ARG; }
-            gi += run;
+    const uint32_t y_idx = qeb.const_slot(p.y);
+    std::vector<int64_t> memo(cs.nodes.size(), -1);
+    // Gate polynomials, Horner in y in constraint-system order.  Circuits multiply whole groups of constraints by one selector
+    // (`q_enable * constraint`), so runs of CONSECUTIVE gates of the form fixed(col, rot) * t_j are folded exactly:
+    //   (..(acc y + f t_1) y + ..) y + f t_r  =  acc y^r + f (t_1 y^(r-1) + .. + t_r)
+    // -- the same field element (distributivity is exact mod r), one multiply per gate less than the term-by-term form.
+    auto selector_split = [&](uint32_t gnode, uint32_t &sel, uint32_t &rest) -> bool {
+        const auto &nd = cs.nodes[gnode];
+        if (nd[0] != N_MUL) return false;
+        for (int side = 0; side < 2; ++side) {
+            const uint32_t a = nd[1 + side], b = nd[2 - side];
+            if (cs.nodes[a][0] == N_FIXED) { sel = a; rest = b; return true; }
         }
-        auto lactive = [&]() { return qeb.sub(qeb.sub(qeb.constant(one), qeb.col(q_llast, 0)), qeb.col(q_lblind, 0)); };
-        if (pk->nsets) {
-            const uint32_t z0 = qeb.col(q_z0, 0), zl = qeb.col(q_z0 + pk->nsets - 1, 0);
-            if (!qpb.scope({{qeb.mul(qeb.sub(qeb.constant(one), z0), qeb.col(q_l0, 0)), ProgramBuilder::HORNER, y_idx}})) return ZKB_ERR_ARG;
-            if (!qpb.scope({{qeb.mul(qeb.sub(qeb.mul(zl, zl), zl), qeb.col(q_llast, 0)), ProgramBuilder::HORNER, y_idx}})) return ZKB_ERR_ARG;
-            for (uint32_t i = 1; i < pk->nsets; ++i) {
-                const uint32_t t = qeb.mul(qeb.sub(qeb.col(q_z0 + i, 0), qeb.col(q_z0 + i - 1, -(int32_t)(bf + 1))), qeb.col(q_l0, 0));
-                if (!qpb.scope({{t, ProgramBuilder::HORNER, y_idx}})) return ZKB_ERR_ARG;
-            }
-            Fr delta_pow = one, delta;
-            {
-                Fr seven = fr_from_u64(7);
-                delta = seven;
-                for (int i = 0; i < 28; ++i) delta = fp_sqr(delta);
-            }
-            for (uint32_t si = 0; si < pk->nsets; ++si) {
-                uint32_t left = qeb.col(q_z0 + si, 1), right = qeb.col(q_z0 + si, 0);
-                for (uint32_t j = si * pk->chunk; j < std::min<size_t>((si + 1) * pk->chunk, cs.perm.size()); ++j) {
-                    const auto &c = cs.perm[j];
-                    const uint32_t vslot = c[0] == N_FIXED ? qsm.fixed0 + c[1] : c[0] == N_ADVICE ? qsm.advice0 + c[1] : qsm.instance0 + c[1];
-                    const uint32_t v = qeb.col(vslot, 0);
-                    left = qeb.mul(left, qeb.add(qeb.add(v, qeb.mul(qeb.col(q_sigma0 + j, 0), qeb.constant(beta))), qeb.constant(gamma)));
-                    right = qeb.mul(right, qeb.add(qeb.add(v, qeb.mul(qeb.col(q_x, 0), qeb.constant(fp_mul(beta, delta_pow)))), qeb.constant(gamma)));
-                    delta_pow = fp_mul(delta_pow, delta);
-                }
-                if (!qpb.scope({{qeb.mul(qeb.sub(left, right), lactive()), ProgramBuilder::HORNER, y_idx}})) { set_error("permutation: %s", qpb.error.c_str()); return ZKB_ERR_ARG; }
-            }
+        return false;
+    };
+    auto same_query = [&](uint32_t a, uint32_t b) { return cs.nodes[a][1] == cs.nodes[b][1] && cs.nodes[a][2] == cs.nodes[b][2]; };
+    for (size_t gi = 0; gi < cs.gates.size();) {
+        uint32_t sel = 0, rest = 0;
+        size_t run = 1;
+        if (selector_split(cs.gates[gi], sel, rest)) {
+            uint32_t s2 = 0, r2 = 0;
+            while (gi + run < cs.gates.size() && run < 4096 && selector_split(cs.gates[gi + run], s2, r2) && same_query(sel, s2)) ++run;
         }
-        for (size_t l = 0; l < nl; ++l) {
-            const CsfLookup &lk = cs.lookups[l];
-            std::vector<uint32_t> fsb;
-            for (auto &inp : lk.inputs) fsb.push_back(qeb.add(compress_exprs(cs, inp, qeb, qsm, s->challenges, memo, theta), qeb.constant(beta)));
-            const uint32_t tb = qeb.add(compress_exprs(cs, lk.table, qeb, qsm, s->challenges, memo, theta), qeb.constant(beta));
-            uint32_t prod = fsb[0];
-            for (size_t j = 1; j < fsb.size(); ++j) prod = qeb.mul(prod, fsb[j]);
-            uint32_t ssum = 0;
-            bool have_sum = false;
-            for (size_t i = 0; i < fsb.size(); ++i) {
-                uint32_t pr = 0;
-                bool have = false;
-                for (size_t j = 0; j < fsb.size(); ++j) {
-                    if (j == i) continue;
-                    pr = have ? qeb.mul(pr, fsb[j]) : fsb[j];
-                    have = true;
-                }
-                if (!have) pr = qeb.constant(one);
-                ssum = have_sum ? qeb.add(ssum, pr) : pr;
-                have_sum = true;
+        if (run < 2) {
+            if (!qpb.scope({{translate(cs, cs.gates[gi], qeb, qsm, challenges, memo), ProgramBuilder::HORNER, y_idx}})) { set_error("gate: %s", qpb.error.c_str()); return ZKB_ERR_ARG; }
+            ++gi;
+            continue;
+        }
+        for (size_t t = 0; t < run; ++t) {
+            uint32_t s2 = 0, r2 = 0;
+            selector_split(cs.gates[gi + t], s2, r2);
+            if (!qpb.scope({{translate(cs, r2, qeb, qsm, challenges, memo), ProgramBuilder::HORNER2, y_idx}})) { set_error("gate: %s", qpb.error.c_str()); return ZKB_ERR_ARG; }
+        }
+        const uint32_t yr_idx = qeb.const_slot(fp_pow_u64(p.y, run));
+        if (!qpb.scope({{translate(cs, sel, qeb, qsm, challenges, memo), ProgramBuilder::FOLD, yr_idx}})) { set_error("gate: %s", qpb.error.c_str()); return ZKB_ERR_ARG; }
+        gi += run;
+    }
+    auto lactive = [&]() { return qeb.sub(qeb.sub(qeb.constant(one), qeb.col(q_llast, 0)), qeb.col(q_lblind, 0)); };
+    if (pk->nsets) {
+        const uint32_t z0 = qeb.col(p.q_z0, 0), zl = qeb.col(p.q_z0 + pk->nsets - 1, 0);
+        if (!qpb.scope({{qeb.mul(qeb.sub(qeb.constant(one), z0), qeb.col(q_l0, 0)), ProgramBuilder::HORNER, y_idx}})) return ZKB_ERR_ARG;
+        if (!qpb.scope({{qeb.mul(qeb.sub(qeb.mul(zl, zl), zl), qeb.col(q_llast, 0)), ProgramBuilder::HORNER, y_idx}})) return ZKB_ERR_ARG;
+        for (uint32_t i = 1; i < pk->nsets; ++i) {
+            const uint32_t t = qeb.mul(qeb.sub(qeb.col(p.q_z0 + i, 0), qeb.col(p.q_z0 + i - 1, -(int32_t)(p.bf + 1))), qeb.col(q_l0, 0));
+            if (!qpb.scope({{t, ProgramBuilder::HORNER, y_idx}})) return ZKB_ERR_ARG;
+        }
+        const Fr delta = perm_delta();
+        Fr delta_pow = one;
+        for (uint32_t si = 0; si < pk->nsets; ++si) {
+            uint32_t left = qeb.col(p.q_z0 + si, 1), right = qeb.col(p.q_z0 + si, 0);
+            for (uint32_t j = si * pk->chunk; j < std::min<size_t>((si + 1) * pk->chunk, cs.perm.size()); ++j) {
+                const uint32_t v = qeb.col(perm_slot(qsm, cs.perm[j]), 0);
+                left = qeb.mul(left, qeb.add(qeb.add(v, qeb.mul(qeb.col(p.q_sigma0 + j, 0), qeb.constant(p.beta))), qeb.constant(p.gamma)));
+                right = qeb.mul(right, qeb.add(qeb.add(v, qeb.mul(qeb.col(q_x, 0), qeb.constant(fp_mul(p.beta, delta_pow)))), qeb.constant(p.gamma)));
+                delta_pow = fp_mul(delta_pow, delta);
             }
-            const uint32_t phi = qeb.col(q_phi0 + (uint32_t)l, 0), phi_next = qeb.col(q_phi0 + (uint32_t)l, 1), m = qeb.col(q_m0 + (uint32_t)l, 0);
-            const uint32_t lhs = qeb.mul(qeb.mul(tb, prod), qeb.sub(phi_next, phi));
-            const uint32_t rhs = qeb.sub(qeb.mul(tb, ssum), qeb.mul(m, prod));
-            std::vector<ProgramBuilder::Root> roots = {{qeb.mul(phi, qeb.col(q_l0, 0)), ProgramBuilder::HORNER, y_idx},
-                                                       {qeb.mul(phi, qeb.col(q_llast, 0)), ProgramBuilder::HORNER, y_idx},
-                                                       {qeb.mul(qeb.sub(lhs, rhs), lactive()), ProgramBuilder::HORNER, y_idx}};
-            if (!qpb.scope(roots)) { set_error("lookup %zu: %s", l, qpb.error.c_str()); return ZKB_ERR_ARG; }
+            if (!qpb.scope({{qeb.mul(qeb.sub(left, right), lactive()), ProgramBuilder::HORNER, y_idx}})) { set_error("permutation: %s", qpb.error.c_str()); return ZKB_ERR_ARG; }
         }
     }
-    // one STOREACC per coset part (the scale constant differs): emit them as separate tiny programs appended at launch
-    std::vector<uint32_t> tinv_idx(pk->E);
-    for (uint32_t j = 0; j < pk->E; ++j) tinv_idx[j] = qeb.const_slot(pk->t_inv[j]);
-    const size_t base_len = qpb.code.size();
-    DeviceProgram qdp;
-    {
-        // device code buffer holds the common body + one trailing STOREACC slot that is rewritten per part
-        qpb.store_acc(0, tinv_idx[0]);
-        ZKB_TRY(upload_program(pool, qpb, qeb, qdp, st));
+    for (size_t l = 0; l < cs.lookups.size(); ++l) {
+        const CsfLookup &lk = cs.lookups[l];
+        std::vector<uint32_t> fsb;
+        for (auto &inp : lk.inputs) fsb.push_back(qeb.add(compress_exprs(cs, inp, qeb, qsm, challenges, memo, p.theta), qeb.constant(p.beta)));
+        const uint32_t tb = qeb.add(compress_exprs(cs, lk.table, qeb, qsm, challenges, memo, p.theta), qeb.constant(p.beta));
+        uint32_t prod = fsb[0];
+        for (size_t j = 1; j < fsb.size(); ++j) prod = qeb.mul(prod, fsb[j]);
+        uint32_t ssum = 0;
+        bool have_sum = false;
+        for (size_t i = 0; i < fsb.size(); ++i) {
+            uint32_t pr = 0;
+            bool have = false;
+            for (size_t j = 0; j < fsb.size(); ++j) {
+                if (j == i) continue;
+                pr = have ? qeb.mul(pr, fsb[j]) : fsb[j];
+                have = true;
+            }
+            if (!have) pr = qeb.constant(one);
+            ssum = have_sum ? qeb.add(ssum, pr) : pr;
+            have_sum = true;
+        }
+        const uint32_t phi = qeb.col(p.q_phi0 + (uint32_t)l, 0), phi_next = qeb.col(p.q_phi0 + (uint32_t)l, 1), m = qeb.col(p.q_m0 + (uint32_t)l, 0);
+        const uint32_t lhs = qeb.mul(qeb.mul(tb, prod), qeb.sub(phi_next, phi));
+        const uint32_t rhs = qeb.sub(qeb.mul(tb, ssum), qeb.mul(m, prod));
+        std::vector<ProgramBuilder::Root> roots = {{qeb.mul(phi, qeb.col(q_l0, 0)), ProgramBuilder::HORNER, y_idx},
+                                                   {qeb.mul(phi, qeb.col(q_llast, 0)), ProgramBuilder::HORNER, y_idx},
+                                                   {qeb.mul(qeb.sub(lhs, rhs), lactive()), ProgramBuilder::HORNER, y_idx}};
+        if (!qpb.scope(roots)) { set_error("lookup %zu: %s", l, qpb.error.c_str()); return ZKB_ERR_ARG; }
     }
+    // one STOREACC per coset part (the scale constant differs): the device code buffer holds the common body + one trailing
+    // STOREACC slot that is rewritten per part
+    p.tinv_idx.resize(pk->E);
+    for (uint32_t j = 0; j < pk->E; ++j) p.tinv_idx[j] = qeb.const_slot(pk->t_inv[j]);
+    p.q_base_len = qpb.code.size();
+    qpb.store_acc(0, p.tinv_idx[0]);
+    return upload_program(p.pool, qpb, qeb, p.qdp, p.st);
+}
 
-    trace.mark("quotient program build+upload");
-    // ---------------------------------------------------------------- evaluate h on the extended domain, part by part
-    Fr *slab, *pows, *h_ext;
+// evaluate h on the extended domain, coset part by coset part: size-n NTTs of every polynomial not in the pk's coset cache, one
+// interpreter launch, x 1/((zeta omega_ext^j)^n - 1)
+static int32_t quotient_evaluate(ProofState &p) {
+    zkb_pk *pk = p.pk;
+    zkb_ctx *ctx = p.ctx;
+    const uint64_t n = p.n;
+    cudaStream_t st = p.st;
+    DevPool &pool = p.pool;
+    const std::vector<Fr *> &qpolys = p.qpolys;
+    Fr *slab, *pows;
     ZKB_TRY(pool.fr(qpolys.size() * n, &slab));
     ZKB_TRY(pool.fr(n, &pows));
-    ZKB_TRY(pool.fr(pk->N, &h_ext));
+    ZKB_TRY(pool.fr(pk->N, &p.h_ext));
     std::vector<Fr *> qcols(qpolys.size());
     for (size_t i = 0; i < qpolys.size(); ++i) qcols[i] = slab + i * n;
     // slots served from the pk's coset cache: fixed [0, nf), sigma, l0 / l_last / l_blind / X
@@ -1471,9 +1468,9 @@ static int32_t prove_finish_impl(zkb_session *s, const uint64_t *z_blinds, const
     std::vector<int> cache_idx(qpolys.size(), -1);
     if (cached) {
         int ci = 0;
-        for (uint32_t i = 0; i < cs.nf; ++i) cache_idx[qsm.fixed0 + i] = ci++;
-        for (size_t i = 0; i < cs.perm.size(); ++i) cache_idx[q_sigma0 + i] = ci++;
-        cache_idx[q_l0] = ci++; cache_idx[q_llast] = ci++; cache_idx[q_lblind] = ci++; cache_idx[q_x] = ci++;
+        for (uint32_t i = 0; i < p.cs.nf; ++i) cache_idx[i] = ci++;
+        for (size_t i = 0; i < p.cs.perm.size(); ++i) cache_idx[p.q_sigma0 + i] = ci++;
+        for (uint32_t i = 0; i < 4; ++i) cache_idx[p.q_l0 + i] = ci++;
     }
     std::vector<Fr *> ntt_src, ntt_dst;
     for (size_t i = 0; i < qpolys.size(); ++i) {
@@ -1481,97 +1478,86 @@ static int32_t prove_finish_impl(zkb_session *s, const uint64_t *z_blinds, const
     }
     Fr **d_qcols = nullptr, **d_hout = nullptr;
     ZKB_TRY(pool.alloc(qcols.size() * sizeof(Fr *) + 8, (void **)&d_qcols));
-    std::vector<Fr *> hout{h_ext};
-    ZKB_TRY(upload_table(pool, hout, &d_hout, st));
     // multi-GPU: coset parts are dealt in contiguous blocks; a rank writes its parts as contiguous n-element rows of h_parts, the rows
     // are all-gathered and interleaved into the extended-domain order h_ext[j + E i] the inverse transform expects
     const Deal dq(ctx, pk->E);
     Fr *h_parts = nullptr;
-    if (dq.on) {
-        ZKB_TRY(pool.fr(dq.padded() * n, &h_parts));
-        std::vector<Fr *> hp{h_parts};
-        ZKB_CUDA(cudaMemcpyAsync(d_hout, hp.data(), sizeof(Fr *), cudaMemcpyHostToDevice, st));
-        ZKB_CUDA(cudaStreamSynchronize(st));
-    }
+    if (dq.on) ZKB_TRY(pool.fr(dq.padded() * n, &h_parts));
+    ZKB_TRY(upload_table(pool, std::vector<Fr *>{dq.on ? h_parts : p.h_ext}, &d_hout, st));
+    const DeviceProgram &qdp = p.qdp;
     for (uint32_t j = 0; j < pk->E; ++j) {
         if (!dq.mine(j)) continue;
-        const Fr gj = fp_mul(pk->zeta, fp_pow_u64(pk->ext_omega, j));
-        ZKB_TRY(fr_powers_device(ctx, gj, n, pows, st));
-        ZKB_TRY(ntt_many(ntt_src, ntt_dst, pk->omega, nullptr, pows));
+        ZKB_TRY(fr_powers_device(ctx, coset_gen(pk, j), n, pows, st));
+        ZKB_TRY(ntt_many(p, ntt_src, ntt_dst, pk->omega, nullptr, pows));
         std::vector<Fr *> cols_j = qcols;
         if (cached)
             for (size_t i = 0; i < qpolys.size(); ++i)
                 if (cache_idx[i] >= 0) cols_j[i] = pk->coset_cache[j][cache_idx[i]];
-        Instr tail{OP_STOREACC, 0, 0, 0, 0u | (tinv_idx[j] << 8)};
+        Instr tail{OP_STOREACC, 0, 0, 0, 0u | (p.tinv_idx[j] << 8)};
         ZKB_CUDA(cudaMemcpyAsync(d_qcols, cols_j.data(), cols_j.size() * sizeof(Fr *), cudaMemcpyHostToDevice, st));
-        ZKB_CUDA(cudaMemcpyAsync(qdp.code + base_len, &tail, sizeof(Instr), cudaMemcpyHostToDevice, st));
-        if (dq.on) ZKB_TRY(expr_run_device(ctx, qdp.code, qdp.ncode, qdp.nregs, d_qcols, qdp.consts, d_hout, k, 1, (uint32_t)((uint64_t)j * n), st));
-        else ZKB_TRY(expr_run_device(ctx, qdp.code, qdp.ncode, qdp.nregs, d_qcols, qdp.consts, d_hout, k, pk->E, j, st));
+        ZKB_CUDA(cudaMemcpyAsync(qdp.code + p.q_base_len, &tail, sizeof(Instr), cudaMemcpyHostToDevice, st));
+        if (dq.on) ZKB_TRY(expr_run_device(ctx, qdp.code, qdp.ncode, qdp.nregs, d_qcols, qdp.consts, d_hout, p.k, 1, (uint32_t)((uint64_t)j * n), st));
+        else ZKB_TRY(expr_run_device(ctx, qdp.code, qdp.ncode, qdp.nregs, d_qcols, qdp.consts, d_hout, p.k, pk->E, j, st));
         ZKB_CUDA(cudaStreamSynchronize(st));  // `tail` and `cols_j` live on the stack
     }
     if (dq.on) {
         ZKB_TRY(deal_gather(ctx, dq, h_parts, n * sizeof(Fr), st));
-        interleave_parts_kernel<<<(unsigned)((pk->N + 255) / 256), 256, 0, st>>>(h_parts, h_ext, k, pk->E);
+        interleave_parts_kernel<<<(unsigned)((pk->N + 255) / 256), 256, 0, st>>>(h_parts, p.h_ext, p.k, pk->E);
         ctx->launches++;
     }
-    trace.mark("quotient: coset NTTs + fused eval");
-    // extended_to_coeff: inverse NTT over the extended domain, 1/N, undo the zeta coset, keep n*(d-1) coefficients
-    ZKB_TRY(ntt_fr_device(ctx, h_ext, h_ext, pk->ext_k, pk->ext_omega_inv, &pk->N_inv, 2, nullptr, st));
-    {
-        std::vector<Fr *> pcs;
-        for (uint32_t i = 0; i < pk->qdeg; ++i) pcs.push_back(h_ext + (size_t)i * n);
-        std::vector<G1Affine> cms;
-        ZKB_TRY(commit_many(pk, pcs, pk->g, n, cms, st));
-        for (auto &cm : cms) ZKB_TRY(tr_write_point(s, cm));
-    }
-    const Fr x = tr_squeeze(s);
-    const Fr xn = fp_pow_u64(x, n);
+    return ZKB_OK;
+}
 
-    trace.mark("extended iNTT + h commits");
-    // ---------------------------------------------------------------- evaluations (prover.rs order)
+// vanishing::construct: extended_to_coeff (inverse NTT over the extended domain, 1/N, undo the zeta coset), the d - 1 pieces of
+// n coefficients, committed with g
+static int32_t quotient_commit(ProofState &p) {
+    zkb_pk *pk = p.pk;
+    ZKB_TRY(ntt_fr_device(p.ctx, p.h_ext, p.h_ext, pk->ext_k, pk->ext_omega_inv, &pk->N_inv, 2, nullptr, p.st));
+    std::vector<Fr *> pieces;
+    for (uint32_t i = 0; i < pk->qdeg; ++i) pieces.push_back(p.h_ext + (size_t)i * p.n);
+    return commit_write(p.s, BASIS_G, pieces, p.st);
+}
+
+// the evaluations written to the transcript (prover.rs order), then the multiopen queries (prover.rs order)
+static int32_t evaluate(ProofState &p) {
+    zkb_pk *pk = p.pk;
+    const Csf &cs = p.cs;
+    const size_t nl = cs.lookups.size();
+    const uint64_t n = p.n;
+    cudaStream_t st = p.st;
     // h(X) = sum_i x^(n i) piece_i
+    const Fr xn = fp_pow_u64(p.x, n);
     Fr *h_poly;
-    ZKB_TRY(pool.fr(n, &h_poly));
+    ZKB_TRY(p.pool.fr(n, &h_poly));
     {
-        std::vector<Fr *> pcs;
+        std::vector<Fr *> pieces;
         std::vector<Fr> cf;
-        Fr cur = one;
-        for (uint32_t i = 0; i < pk->qdeg; ++i) { pcs.push_back(h_ext + (size_t)i * n); cf.push_back(cur); cur = fp_mul(cur, xn); }
-        Fr **d_p = nullptr;
-        Fr *d_c = nullptr;
-        ZKB_TRY(upload_table(pool, pcs, &d_p, st));
-        ZKB_TRY(pool.fr(cf.size(), &d_c));
-        ZKB_CUDA(cudaMemcpyAsync(d_c, cf.data(), cf.size() * sizeof(Fr), cudaMemcpyHostToDevice, st));
-        ZKB_TRY(lincomb_device(ctx, d_p, d_c, (uint32_t)pcs.size(), n, h_poly, false, st));
+        Fr cur = Fr::one();
+        for (uint32_t i = 0; i < pk->qdeg; ++i) { pieces.push_back(p.h_ext + (size_t)i * n); cf.push_back(cur); cur = fp_mul(cur, xn); }
+        ZKB_TRY(lincomb(p.s, pieces, cf, h_poly, false, st));
         ZKB_CUDA(cudaStreamSynchronize(st));
     }
-    std::vector<OpenQuery> queries;
-    int next_id = 0;
-    std::vector<int> adv_id(cs.na), fix_id(cs.nf), sig_id(cs.perm.size()), z_id(pk->nsets), phi_id(nl), m_id(nl);
-    for (auto &v : adv_id) v = next_id++;
-    for (auto &v : fix_id) v = next_id++;
-    for (auto &v : sig_id) v = next_id++;
-    for (auto &v : z_id) v = next_id++;
-    for (auto &v : phi_id) v = next_id++;
-    for (auto &v : m_id) v = next_id++;
+    int next_id = 0;   // identities of the committed polynomials, in this order
+    auto ids = [&](size_t count) { std::vector<int> v(count); for (auto &e : v) e = next_id++; return v; };
+    const std::vector<int> adv_id = ids(cs.na), fix_id = ids(cs.nf), sig_id = ids(cs.perm.size()), z_id = ids(pk->nsets), phi_id = ids(nl), m_id = ids(nl);
     const int h_id = next_id++, rand_id = next_id++;
-    const int64_t rot_last = -(int64_t)(bf + 1);
-    // (1) the evaluations written to the transcript, in order; `queries` is built afterwards in the multiopen order
+    const int64_t rot_last = -(int64_t)(p.bf + 1);
+    // (1) the evaluations written to the transcript, in order; the queries are built afterwards in the multiopen order
     struct EvalReq { int poly_id; const Fr *poly; int64_t rot; };
     std::vector<EvalReq> reqs;
-    for (auto &q : cs.advq) reqs.push_back({adv_id[q[0]], adv_polys[q[0]], q[1]});
+    for (auto &q : cs.advq) reqs.push_back({adv_id[q[0]], p.adv_polys[q[0]], q[1]});
     for (auto &q : cs.fixq) reqs.push_back({fix_id[q[0]], pk->fixed_polys[q[0]], q[1]});
-    reqs.push_back({rand_id, random_poly, 0});
+    reqs.push_back({rand_id, p.random_poly, 0});
     for (size_t i = 0; i < cs.perm.size(); ++i) reqs.push_back({sig_id[i], pk->sigma_polys[i], 0});
     for (uint32_t i = 0; i < pk->nsets; ++i) {
-        reqs.push_back({z_id[i], z_polys[i], 0});
-        reqs.push_back({z_id[i], z_polys[i], 1});
-        if (i + 1 != pk->nsets) reqs.push_back({z_id[i], z_polys[i], rot_last});
+        reqs.push_back({z_id[i], p.z_polys[i], 0});
+        reqs.push_back({z_id[i], p.z_polys[i], 1});
+        if (i + 1 != pk->nsets) reqs.push_back({z_id[i], p.z_polys[i], rot_last});
     }
     for (size_t l = 0; l < nl; ++l) {
-        reqs.push_back({phi_id[l], phi_polys[l], 0});
-        reqs.push_back({phi_id[l], phi_polys[l], 1});
-        reqs.push_back({m_id[l], m_polys[l], 0});
+        reqs.push_back({phi_id[l], p.phi_polys[l], 0});
+        reqs.push_back({phi_id[l], p.phi_polys[l], 1});
+        reqs.push_back({m_id[l], p.m_polys[l], 0});
     }
     const size_t n_written = reqs.size();
     reqs.push_back({h_id, h_poly, 0});  // needed by SHPLONK, not written
@@ -1579,209 +1565,211 @@ static int32_t prove_finish_impl(zkb_session *s, const uint64_t *z_blinds, const
     std::map<int64_t, std::vector<size_t>> by_rot;
     for (size_t i = 0; i < reqs.size(); ++i) by_rot[reqs[i].rot].push_back(i);
     std::vector<Fr> evals(reqs.size());
-    std::map<int64_t, Fr> point_of;
     for (auto &kv : by_rot) {
-        const Fr pt = fp_mul(x, fr_pow_i64(pk->omega, pk->omega_inv, kv.first));
-        point_of[kv.first] = pt;
+        const Fr pt = fp_mul(p.x, fr_pow_i64(pk->omega, pk->omega_inv, kv.first));
+        p.point_of[kv.first] = pt;
         std::vector<Fr *> ptrs;
         for (size_t i : kv.second) ptrs.push_back(const_cast<Fr *>(reqs[i].poly));
         Fr **d_p = nullptr;
-        ZKB_TRY(upload_table(pool, ptrs, &d_p, st));
+        ZKB_TRY(upload_table(p.pool, ptrs, &d_p, st));
         // multi-GPU: the polynomials of a rotation are dealt, the 32-byte results all-gathered
-        const Deal de(ctx, ptrs.size());
+        const Deal de(p.ctx, ptrs.size());
         std::vector<Fr> res(std::max<size_t>(1, de.padded()));
-        if (!de.on) {
-            ZKB_TRY(poly_eval_device(ctx, d_p, (uint32_t)ptrs.size(), n, pt, res.data(), st));
-        } else {
-            const size_t lo = (size_t)de.rank * de.blk, hi = std::min(ptrs.size(), lo + de.blk);
-            if (hi > lo) ZKB_TRY(poly_eval_device(ctx, d_p + lo, (uint32_t)(hi - lo), n, pt, res.data() + lo, st));
-            Fr *d_r = nullptr;
-            ZKB_TRY(scratch_get(ctx, SCR_COMM, de.padded() * sizeof(Fr), (void **)&d_r));
-            ZKB_CUDA(cudaMemcpyAsync(d_r + lo, res.data() + lo, de.blk * sizeof(Fr), cudaMemcpyHostToDevice, st));
-            ZKB_TRY(deal_gather(ctx, de, d_r, sizeof(Fr), st));
-            ZKB_CUDA(cudaMemcpyAsync(res.data(), d_r, de.padded() * sizeof(Fr), cudaMemcpyDeviceToHost, st));
-            ZKB_CUDA(cudaStreamSynchronize(st));
-        }
+        const size_t lo = de.first(), hi = std::min(ptrs.size(), lo + de.blk);
+        if (hi > lo) ZKB_TRY(poly_eval_device(p.ctx, d_p + lo, (uint32_t)(hi - lo), n, pt, res.data() + lo, st));
+        ZKB_TRY(deal_gather_host(p.ctx, de, res.data(), sizeof(Fr), st));
         for (size_t t = 0; t < kv.second.size(); ++t) evals[kv.second[t]] = res[t];
     }
-    for (size_t i = 0; i < n_written; ++i) tr_write_scalar(s, evals[i]);
-    std::map<std::pair<int, int64_t>, Fr> eval_of;
-    for (size_t i = 0; i < reqs.size(); ++i) eval_of[{reqs[i].poly_id, reqs[i].rot}] = evals[i];
+    for (size_t i = 0; i < n_written; ++i) p.s->tr.write_scalar(evals[i]);
+    for (size_t i = 0; i < reqs.size(); ++i) p.eval_of[{reqs[i].poly_id, reqs[i].rot}] = evals[i];
 
     // (2) multiopen queries in prover.rs order
-    auto push_q = [&](int id, const Fr *poly, int64_t rot) { queries.push_back({id, poly, rot, point_of[rot], eval_of[{id, rot}]}); };
-    for (auto &q : cs.advq) push_q(adv_id[q[0]], adv_polys[q[0]], q[1]);
-    for (uint32_t i = 0; i < pk->nsets; ++i) { push_q(z_id[i], z_polys[i], 0); push_q(z_id[i], z_polys[i], 1); }
-    for (int i = (int)pk->nsets - 2; i >= 0; --i) push_q(z_id[i], z_polys[i], rot_last);
-    for (size_t l = 0; l < nl; ++l) { push_q(phi_id[l], phi_polys[l], 0); push_q(phi_id[l], phi_polys[l], 1); push_q(m_id[l], m_polys[l], 0); }
+    auto push_q = [&](int id, const Fr *poly, int64_t rot) { p.queries.push_back({id, poly, rot, p.point_of[rot], p.eval_of[{id, rot}]}); };
+    for (auto &q : cs.advq) push_q(adv_id[q[0]], p.adv_polys[q[0]], q[1]);
+    for (uint32_t i = 0; i < pk->nsets; ++i) { push_q(z_id[i], p.z_polys[i], 0); push_q(z_id[i], p.z_polys[i], 1); }
+    for (int i = (int)pk->nsets - 2; i >= 0; --i) push_q(z_id[i], p.z_polys[i], rot_last);
+    for (size_t l = 0; l < nl; ++l) { push_q(phi_id[l], p.phi_polys[l], 0); push_q(phi_id[l], p.phi_polys[l], 1); push_q(m_id[l], p.m_polys[l], 0); }
     for (auto &q : cs.fixq) push_q(fix_id[q[0]], pk->fixed_polys[q[0]], q[1]);
     for (size_t i = 0; i < cs.perm.size(); ++i) push_q(sig_id[i], pk->sigma_polys[i], 0);
     push_q(h_id, h_poly, 0);
-    push_q(rand_id, random_poly, 0);
+    push_q(rand_id, p.random_poly, 0);
+    return ZKB_OK;
+}
 
-    trace.mark("evaluations");
-    // ---------------------------------------------------------------- SHPLONK (multiopen/shplonk/prover.rs)
-    const Fr sy = tr_squeeze(s);
-    // construct_intermediate_sets
-    struct Commit { int id; const Fr *poly; std::vector<int64_t> rots; };
-    std::vector<Commit> cmap;
-    std::vector<int64_t> super_rots;
-    for (auto &q : queries) {
-        if (std::find(super_rots.begin(), super_rots.end(), q.rot) == super_rots.end()) super_rots.push_back(q.rot);
-        auto it = std::find_if(cmap.begin(), cmap.end(), [&](const Commit &c) { return c.id == q.poly_id; });
+// low-degree interpolant through (points, evals): coefficients, low to high
+static std::vector<Fr> interpolate(const std::vector<Fr> &pts, const std::vector<Fr> &evs) {
+    const size_t m = pts.size();
+    std::vector<Fr> coeffs(m, Fr::zero());
+    for (size_t j = 0; j < m; ++j) {
+        std::vector<Fr> num{Fr::one()};
+        Fr den = Fr::one();
+        for (size_t t = 0; t < m; ++t) {
+            if (t == j) continue;
+            std::vector<Fr> nx(num.size() + 1, Fr::zero());
+            for (size_t i = 0; i < num.size(); ++i) {
+                nx[i + 1] = fp_add(nx[i + 1], num[i]);
+                nx[i] = fp_sub(nx[i], fp_mul(pts[t], num[i]));
+            }
+            num.swap(nx);
+            den = fp_mul(den, fp_sub(pts[j], pts[t]));
+        }
+        const Fr sc = fp_mul(evs[j], fp_inv(den));
+        for (size_t i = 0; i < m; ++i) coeffs[i] = fp_add(coeffs[i], fp_mul(num[i], sc));
+    }
+    return coeffs;
+}
+static Fr horner_host(const std::vector<Fr> &c, const Fr &at) {
+    Fr acc = Fr::zero();
+    for (size_t i = c.size(); i-- > 0;) acc = fp_add(fp_mul(acc, at), c[i]);
+    return acc;
+}
+
+// multiopen/shplonk/prover.rs up to the commitment of h_x: construct_intermediate_sets, then per rotation set
+// Q_i = (sum_j y^j (P_ij - R_ij)) / Z_i and h_x = sum_i v^i Q_i
+static int32_t shplonk_commit_h(ProofState &p) {
+    zkb_session *s = p.s;
+    const uint64_t n = p.n;
+    cudaStream_t st = p.st;
+    const Fr one = Fr::one();
+    // construct_intermediate_sets: points sorted by canonical value, commitments and sets by first appearance
+    std::vector<ShplonkCommit> &cmap = p.sh_commits;
+    for (auto &q : p.queries) {
+        if (std::find(p.super_rots.begin(), p.super_rots.end(), q.rot) == p.super_rots.end()) p.super_rots.push_back(q.rot);
+        auto it = std::find_if(cmap.begin(), cmap.end(), [&](const ShplonkCommit &c) { return c.id == q.poly_id; });
         if (it == cmap.end()) cmap.push_back({q.poly_id, q.poly, {q.rot}});
         else if (std::find(it->rots.begin(), it->rots.end(), q.rot) == it->rots.end()) it->rots.push_back(q.rot);
     }
-    auto sort_rots = [&](std::vector<int64_t> &r) { std::sort(r.begin(), r.end(), [&](int64_t a, int64_t b) { return fr_less(point_of[a], point_of[b]); }); };
-    sort_rots(super_rots);
+    auto sort_rots = [&](std::vector<int64_t> &r) { std::sort(r.begin(), r.end(), [&](int64_t a, int64_t b) { return fr_less(p.point_of[a], p.point_of[b]); }); };
+    sort_rots(p.super_rots);
     for (auto &c : cmap) sort_rots(c.rots);
-    struct RSet { std::vector<int64_t> rots; std::vector<Commit *> comms; };
-    std::vector<RSet> rsets;
     for (auto &c : cmap) {
-        auto it = std::find_if(rsets.begin(), rsets.end(), [&](const RSet &r) { return r.rots == c.rots; });
-        if (it == rsets.end()) rsets.push_back({c.rots, {&c}});
+        auto it = std::find_if(p.rsets.begin(), p.rsets.end(), [&](const RotationSet &r) { return r.rots == c.rots; });
+        if (it == p.rsets.end()) p.rsets.push_back({c.rots, {&c}, {}, {}});
         else it->comms.push_back(&c);
     }
-    const Fr sv = tr_squeeze(s);
-    // low-degree interpolant through (points, evals): coefficients, low to high
-    auto interpolate = [&](const std::vector<Fr> &pts, const std::vector<Fr> &evs) {
-        const size_t m = pts.size();
-        std::vector<Fr> coeffs(m, Fr::zero());
-        for (size_t j = 0; j < m; ++j) {
-            std::vector<Fr> num{one};
-            Fr den = one;
-            for (size_t t = 0; t < m; ++t) {
-                if (t == j) continue;
-                std::vector<Fr> nx(num.size() + 1, Fr::zero());
-                for (size_t i = 0; i < num.size(); ++i) {
-                    nx[i + 1] = fp_add(nx[i + 1], num[i]);
-                    nx[i] = fp_sub(nx[i], fp_mul(pts[t], num[i]));
-                }
-                num.swap(nx);
-                den = fp_mul(den, fp_sub(pts[j], pts[t]));
-            }
-            const Fr sc = fp_mul(evs[j], fp_inv(den));
-            for (size_t i = 0; i < m; ++i) coeffs[i] = fp_add(coeffs[i], fp_mul(num[i], sc));
-        }
-        return coeffs;
-    };
-    auto horner_host = [&](const std::vector<Fr> &c, const Fr &at) {
-        Fr acc = Fr::zero();
-        for (size_t i = c.size(); i-- > 0;) acc = fp_add(fp_mul(acc, at), c[i]);
-        return acc;
-    };
-    Fr *hx, *work, *work2, *d_small;
-    ZKB_TRY(pool.fr(n, &hx));
-    ZKB_TRY(pool.fr(n, &work));
-    ZKB_TRY(pool.fr(n, &work2));
-    ZKB_TRY(pool.fr(256, &d_small));
-    ZKB_CUDA(cudaMemsetAsync(hx, 0, n * sizeof(Fr), st));
-    struct SetData { std::vector<Fr> pts; std::vector<std::vector<Fr>> r_coeffs; };
-    std::vector<SetData> sdata(rsets.size());
-    {
-        Fr vpow = one;
-        for (size_t si = 0; si < rsets.size(); ++si) {
-            RSet &rs = rsets[si];
-            SetData &sd = sdata[si];
-            for (int64_t r : rs.rots) sd.pts.push_back(point_of[r]);
-            ZKB_ARG(sd.pts.size() <= 256);   // Keccak's hot cell column is opened at 56 rotations (keccak_packed_multi.rs:59-68)
-            // N_i(X) = sum_j y^j (P_ij(X) - R_ij(X))
-            std::vector<Fr *> ptrs;
-            std::vector<Fr> cf;
-            std::vector<Fr> rsum(sd.pts.size(), Fr::zero());
-            Fr ypow = one;
-            for (Commit *c : rs.comms) {
-                std::vector<Fr> evs;
-                for (int64_t r : rs.rots) evs.push_back(eval_of[{c->id, r}]);
-                sd.r_coeffs.push_back(interpolate(sd.pts, evs));
-                for (size_t i = 0; i < sd.pts.size(); ++i) rsum[i] = fp_add(rsum[i], fp_mul(sd.r_coeffs.back()[i], ypow));
-                ptrs.push_back(const_cast<Fr *>(c->poly));
-                cf.push_back(ypow);
-                ypow = fp_mul(ypow, sy);
-            }
-            Fr **d_p = nullptr;
-            Fr *d_c = nullptr;
-            ZKB_TRY(upload_table(pool, ptrs, &d_p, st));
-            ZKB_TRY(pool.fr(cf.size(), &d_c));
-            ZKB_CUDA(cudaMemcpyAsync(d_c, cf.data(), cf.size() * sizeof(Fr), cudaMemcpyHostToDevice, st));
-            ZKB_TRY(lincomb_device(ctx, d_p, d_c, (uint32_t)ptrs.size(), n, work, false, st));
-            ZKB_CUDA(cudaMemcpyAsync(d_small, rsum.data(), rsum.size() * sizeof(Fr), cudaMemcpyHostToDevice, st));
-            sub_low_kernel<<<1, 256, 0, st>>>(work, d_small, (uint32_t)rsum.size());
-            ctx->launches++;
-            ZKB_CUDA(cudaStreamSynchronize(st));
-            // divide by the vanishing polynomial of the set, one root at a time
-            Fr *src = work, *dst = work2;
-            for (const Fr &p : sd.pts) {
-                ZKB_TRY(kate_division_device(ctx, src, n, p, dst, st));
-                std::swap(src, dst);
-            }
-            // h_x += v^i * Q_i
-            std::vector<Fr *> one_ptr{src};
-            Fr **d_q = nullptr;
-            Fr *d_v = nullptr;
-            ZKB_TRY(upload_table(pool, one_ptr, &d_q, st));
-            ZKB_TRY(pool.fr(1, &d_v));
-            ZKB_CUDA(cudaMemcpyAsync(d_v, &vpow, sizeof(Fr), cudaMemcpyHostToDevice, st));
-            ZKB_TRY(lincomb_device(ctx, d_q, d_v, 1, n, hx, true, st));
-            ZKB_CUDA(cudaStreamSynchronize(st));
-            vpow = fp_mul(vpow, sv);
-        }
-    }
-    {
-        G1Affine cm;
-        { std::vector<Fr *> one_col{hx}; std::vector<G1Affine> r1; ZKB_TRY(commit_many(pk, one_col, pk->g, n, r1, st)); cm = r1[0]; }
-        ZKB_TRY(tr_write_point(s, cm));
-    }
-    const Fr su = tr_squeeze(s);
-    {
-        // L(X) = sum_i v^i z_i sum_j y^j (P_ij(X) - r_ij) - zt * h_x(X), scaled by 1/z_0, divided by (X - u)
-        std::vector<Fr> super_pts;
-        for (int64_t r : super_rots) super_pts.push_back(point_of[r]);
-        std::vector<Fr> zdiff(rsets.size());
-        for (size_t si = 0; si < rsets.size(); ++si) {
-            Fr z = one;
-            for (size_t t = 0; t < super_rots.size(); ++t) {
-                if (std::find(rsets[si].rots.begin(), rsets[si].rots.end(), super_rots[t]) == rsets[si].rots.end()) z = fp_mul(z, fp_sub(su, super_pts[t]));
-            }
-            zdiff[si] = z;
-        }
-        Fr zt = one;
-        for (auto &p : super_pts) zt = fp_mul(zt, fp_sub(su, p));
-        const Fr z0inv = fp_inv(zdiff[0]);
+    ZKB_TRY(p.pool.fr(n, &p.hx));
+    ZKB_TRY(p.pool.fr(n, &p.work));
+    ZKB_TRY(p.pool.fr(n, &p.work2));
+    ZKB_TRY(p.pool.fr(256, &p.d_small));
+    ZKB_CUDA(cudaMemsetAsync(p.hx, 0, n * sizeof(Fr), st));
+    Fr vpow = one;
+    for (RotationSet &rs : p.rsets) {
+        for (int64_t r : rs.rots) rs.pts.push_back(p.point_of[r]);
+        ZKB_ARG(rs.pts.size() <= 256);   // Keccak's hot cell column is opened at 56 rotations (keccak_packed_multi.rs:59-68)
+        // N_i(X) = sum_j y^j (P_ij(X) - R_ij(X))
         std::vector<Fr *> ptrs;
         std::vector<Fr> cf;
-        Fr const_term = Fr::zero();
-        Fr vpow = one;
-        for (size_t si = 0; si < rsets.size(); ++si) {
-            Fr ypow = one;
-            for (size_t ci = 0; ci < rsets[si].comms.size(); ++ci) {
-                const Fr w = fp_mul(fp_mul(fp_mul(vpow, zdiff[si]), ypow), z0inv);
-                ptrs.push_back(const_cast<Fr *>(rsets[si].comms[ci]->poly));
-                cf.push_back(w);
-                const_term = fp_add(const_term, fp_mul(w, horner_host(sdata[si].r_coeffs[ci], su)));
-                ypow = fp_mul(ypow, sy);
-            }
-            vpow = fp_mul(vpow, sv);
+        std::vector<Fr> rsum(rs.pts.size(), Fr::zero());
+        Fr ypow = one;
+        for (const ShplonkCommit *c : rs.comms) {
+            std::vector<Fr> evs;
+            for (int64_t r : rs.rots) evs.push_back(p.eval_of[{c->id, r}]);
+            rs.r_coeffs.push_back(interpolate(rs.pts, evs));
+            for (size_t i = 0; i < rs.pts.size(); ++i) rsum[i] = fp_add(rsum[i], fp_mul(rs.r_coeffs.back()[i], ypow));
+            ptrs.push_back(const_cast<Fr *>(c->poly));
+            cf.push_back(ypow);
+            ypow = fp_mul(ypow, p.sy);
         }
-        ptrs.push_back(hx);
-        cf.push_back(fp_neg(fp_mul(zt, z0inv)));
-        Fr **d_p = nullptr;
-        Fr *d_c = nullptr;
-        ZKB_TRY(upload_table(pool, ptrs, &d_p, st));
-        ZKB_TRY(pool.fr(cf.size(), &d_c));
-        ZKB_CUDA(cudaMemcpyAsync(d_c, cf.data(), cf.size() * sizeof(Fr), cudaMemcpyHostToDevice, st));
-        ZKB_TRY(lincomb_device(ctx, d_p, d_c, (uint32_t)ptrs.size(), n, work, false, st));
-        ZKB_CUDA(cudaMemcpyAsync(d_small, &const_term, sizeof(Fr), cudaMemcpyHostToDevice, st));
-        sub_low_kernel<<<1, 256, 0, st>>>(work, d_small, 1);
-        ctx->launches++;
+        ZKB_TRY(lincomb(s, ptrs, cf, p.work, false, st));
+        ZKB_CUDA(cudaMemcpyAsync(p.d_small, rsum.data(), rsum.size() * sizeof(Fr), cudaMemcpyHostToDevice, st));
+        sub_low_kernel<<<1, 256, 0, st>>>(p.work, p.d_small, (uint32_t)rsum.size());
+        p.ctx->launches++;
         ZKB_CUDA(cudaStreamSynchronize(st));
-        ZKB_TRY(kate_division_device(ctx, work, n, su, work2, st));
-        G1Affine cm;
-        { std::vector<Fr *> one_col{work2}; std::vector<G1Affine> r1; ZKB_TRY(commit_many(pk, one_col, pk->g, n, r1, st)); cm = r1[0]; }
-        ZKB_TRY(tr_write_point(s, cm));
+        // divide by the vanishing polynomial of the set, one root at a time
+        Fr *src = p.work, *dst = p.work2;
+        for (const Fr &pt : rs.pts) {
+            ZKB_TRY(kate_division_device(p.ctx, src, n, pt, dst, st));
+            std::swap(src, dst);
+        }
+        // h_x += v^i * Q_i
+        const std::vector<Fr> vcoef{vpow};
+        ZKB_TRY(lincomb(s, {src}, vcoef, p.hx, true, st));
+        ZKB_CUDA(cudaStreamSynchronize(st));
+        vpow = fp_mul(vpow, p.sv);
     }
+    return commit_write(s, BASIS_G, {p.hx}, st);
+}
+
+// multiopen/shplonk/prover.rs after u: L(X) = sum_i v^i z_i sum_j y^j (P_ij(X) - r_ij(u)) - zt h_x(X), scaled by 1/z_0, divided by
+// (X - u), committed with g
+static int32_t shplonk_open(ProofState &p) {
+    const Fr one = Fr::one();
+    cudaStream_t st = p.st;
+    const std::vector<RotationSet> &rsets = p.rsets;
+    std::vector<Fr> super_pts;
+    for (int64_t r : p.super_rots) super_pts.push_back(p.point_of[r]);
+    std::vector<Fr> zdiff(rsets.size());
+    for (size_t si = 0; si < rsets.size(); ++si) {
+        Fr z = one;
+        for (size_t t = 0; t < p.super_rots.size(); ++t) {
+            if (std::find(rsets[si].rots.begin(), rsets[si].rots.end(), p.super_rots[t]) == rsets[si].rots.end()) z = fp_mul(z, fp_sub(p.su, super_pts[t]));
+        }
+        zdiff[si] = z;
+    }
+    Fr zt = one;
+    for (auto &pt : super_pts) zt = fp_mul(zt, fp_sub(p.su, pt));
+    const Fr z0inv = fp_inv(zdiff[0]);
+    std::vector<Fr *> ptrs;
+    std::vector<Fr> cf;
+    Fr const_term = Fr::zero();
+    Fr vpow = one;
+    for (size_t si = 0; si < rsets.size(); ++si) {
+        Fr ypow = one;
+        for (size_t ci = 0; ci < rsets[si].comms.size(); ++ci) {
+            const Fr w = fp_mul(fp_mul(fp_mul(vpow, zdiff[si]), ypow), z0inv);
+            ptrs.push_back(const_cast<Fr *>(rsets[si].comms[ci]->poly));
+            cf.push_back(w);
+            const_term = fp_add(const_term, fp_mul(w, horner_host(rsets[si].r_coeffs[ci], p.su)));
+            ypow = fp_mul(ypow, p.sy);
+        }
+        vpow = fp_mul(vpow, p.sv);
+    }
+    ptrs.push_back(p.hx);
+    cf.push_back(fp_neg(fp_mul(zt, z0inv)));
+    ZKB_TRY(lincomb(p.s, ptrs, cf, p.work, false, st));
+    ZKB_CUDA(cudaMemcpyAsync(p.d_small, &const_term, sizeof(Fr), cudaMemcpyHostToDevice, st));
+    sub_low_kernel<<<1, 256, 0, st>>>(p.work, p.d_small, 1);
+    p.ctx->launches++;
+    ZKB_CUDA(cudaStreamSynchronize(st));
+    ZKB_TRY(kate_division_device(p.ctx, p.work, p.n, p.su, p.work2, st));
+    return commit_write(p.s, BASIS_G, {p.work2}, st);
+}
+
+// create_proof after the advice phases.  Every transcript squeeze happens here, so this function reads as the transcript order.
+static int32_t prove_finish_impl(zkb_session *s, const uint64_t *z_blinds, const uint64_t *phi_blinds, const uint64_t *random_poly_host) {
+    ProofState p(s);
+    Transcript &tr = s->tr;
+    StageTrace trace(p.st);
+    p.theta = tr.squeeze();
+    ZKB_TRY(lookups_prepare(p));
+    trace.mark("lookups: compress + m + commit");
+    p.beta = tr.squeeze();
+    p.gamma = tr.squeeze();
+    ZKB_TRY(permutation_commit(p, z_blinds));
+    trace.mark("permutation z + commit");
+    ZKB_TRY(lookups_commit_sums(p, phi_blinds));
+    trace.mark("lookup phi + commit");
+    ZKB_TRY(vanishing_commit_random(p, random_poly_host));
+    p.y = tr.squeeze();
+    trace.mark("random poly commit");
+    ZKB_TRY(to_coefficients(p));
+    trace.mark("lagrange_to_coeff (all columns)");
+    ZKB_TRY(quotient_program(p));
+    trace.mark("quotient program build+upload");
+    ZKB_TRY(quotient_evaluate(p));
+    trace.mark("quotient: coset NTTs + fused eval");
+    ZKB_TRY(quotient_commit(p));
+    p.x = tr.squeeze();
+    trace.mark("extended iNTT + h commits");
+    ZKB_TRY(evaluate(p));
+    trace.mark("evaluations");
+    p.sy = tr.squeeze();
+    p.sv = tr.squeeze();
+    ZKB_TRY(shplonk_commit_h(p));
+    p.su = tr.squeeze();
+    ZKB_TRY(shplonk_open(p));
     trace.mark("shplonk");
-    if (s->cb_error) { set_error("the caller's transcript callback failed (%d)", s->cb_error); return ZKB_ERR_STATE; }
+    ZKB_TRY(tr.status());
     s->finished = true;
     return ZKB_OK;
 }
@@ -1801,11 +1789,12 @@ extern "C" int32_t zkb_prove_finish(zkb_session *s, const uint64_t *z_blinds, co
         ZKB_CUDA(cudaSetDevice(pk->ctx->device));
         ZKB_TRY(prove_finish_impl(s, z_blinds, phi_blinds, random_poly));
     }
-    *proof_len = s->proof.size();
+    const std::vector<uint8_t> &proof = s->tr.proof;
+    *proof_len = proof.size();
     if (proof_out) {
-        if (proof_cap < s->proof.size()) { set_error("zkb_prove_finish: buffer of %llu bytes, proof has %llu (kept in the session: call again)",
-                                                     (unsigned long long)proof_cap, (unsigned long long)s->proof.size()); return ZKB_ERR_ARG; }
-        memcpy(proof_out, s->proof.data(), s->proof.size());
+        if (proof_cap < proof.size()) { set_error("zkb_prove_finish: buffer of %llu bytes, proof has %llu (kept in the session: call again)",
+                                                  (unsigned long long)proof_cap, (unsigned long long)proof.size()); return ZKB_ERR_ARG; }
+        memcpy(proof_out, proof.data(), proof.size());
     }
     return ZKB_OK;
 }
