@@ -15,8 +15,9 @@
  *     so Rust passes `slice.as_ptr()` with no conversion.
  *   - `*_host` entry points take HOST pointers and include the H2D / D2H copies; `*_dev` take DEVICE pointers and a
  *     CUDA stream (as void*, NULL = the context's stream) and never synchronise unless stated.
- *   - opaque handles are created / destroyed explicitly; one proof at a time per context (the reference serialises
- *     proving behind a Mutex<Prover>: prover/src/test/inner.rs:20-30).
+ *   - opaque handles are created / destroyed explicitly; one proving session at a time per context (the reference serialises
+ *     proving behind a Mutex<Prover>: prover/src/test/inner.rs:20-30); one session may prove several circuits
+ *     (zkb_prove_begin_multi).
  *   - There is NO CPU fallback: without a CUDA device every compute entry point fails with ZKB_ERR_CUDA.
  */
 #ifndef ZKB200_H
@@ -215,7 +216,16 @@ ZKB_API int32_t zkb_comm_destroy(zkb_ctx *ctx);
  *                    too short (ZKB_ERR_ARG, *proof_len set) -- call again with a buffer of *proof_len bytes; later calls only copy.
  *                    Multi-GPU sessions (zkb_comm_init): every zkb_pk_* / zkb_prove_* call, zkb_pk_vk_bytes included, is a COLLECTIVE
  *                    over the communicator and must be issued by all ranks in the same order; a rank-local failure (allocation, CUDA
- *                    error) leaves the other ranks inside a collective, so abort the job on any non-zero return.                  */
+ *                    error) leaves the other ranks inside a collective, so abort the job on any non-zero return.
+ * zkb_prove_begin_multi  create_proof's `circuits: &[C]`: one proof of C >= 1 circuits under one proving key.  They share the
+ *                    challenges, one quotient h (every circuit's constraints continue the same Horner chain in y), the random
+ *                    polynomial and one SHPLONK opening.  Everything per circuit is CIRCUIT-MAJOR: instance_values / instance_lens hold
+ *                    C * num_instance columns (circuit c's column i at c * num_instance + i); zkb_prove_advice_phase takes C * num_advice
+ *                    pointers (circuit c's column j at c * num_advice + j); zkb_prove_upload_advice takes that same index; zkb_prove_finish
+ *                    takes z_blinds [C][n_sets][bf], phi_blinds [C][n_lookups][bf] and ONE random_poly [n].  transcript_kind 0, 1, 2 as
+ *                    zkb_prove_begin_ex (vt must be NULL), 3 = the caller's transcript through vt as zkb_prove_begin_cb.  num_circuits = 0
+ *                    is ZKB_ERR_ARG; running out of device memory at any stage is ZKB_ERR_ALLOC.  The other zkb_prove_begin* entry
+ *                    points are C = 1 and C = 1 here gives the same bytes as they do.                                                */
 typedef struct zkb_pk zkb_pk;
 typedef struct zkb_session zkb_session;
 ZKB_API int32_t zkb_pk_create(zkb_ctx *ctx, const uint32_t *csf, uint64_t csf_words, const uint64_t *const *fixed_values,
@@ -265,6 +275,10 @@ typedef struct zkb_transcript_vtable {
 } zkb_transcript_vtable;
 ZKB_API int32_t zkb_prove_begin_cb(zkb_pk *pk, const zkb_transcript_vtable *vt, const uint64_t transcript_repr[4],
                                    const uint64_t *const *instance_values, const uint32_t *instance_lens, zkb_session **out);
+/* num_circuits circuits in one proof; see "zkb_prove_begin_multi" above zkb_pk_create.  (ABI 1.2) */
+ZKB_API int32_t zkb_prove_begin_multi(zkb_pk *pk, int32_t transcript_kind, const zkb_transcript_vtable *vt,
+                                      const uint64_t transcript_repr[4], uint32_t num_circuits,
+                                      const uint64_t *const *instance_values, const uint32_t *instance_lens, zkb_session **out);
 /* Host-only transcript primitives (no CUDA device needed; used by the CPU test-suite to pin the session's hashers):
  * zkb_poseidon_hash_host        absorb n Fr (Montgomery) into a fresh PoseidonTranscript sponge, squeeze one challenge
  * zkb_blake2b_challenge_host    feed bytes to a fresh Blake2b("Halo2-Transcript") state, squeeze one Challenge255 (mod r)

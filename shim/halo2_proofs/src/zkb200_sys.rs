@@ -49,6 +49,8 @@ extern "C" {
                               out: *mut *mut zkb_session) -> i32;
     pub fn zkb_prove_begin_cb(pk: *mut zkb_pk, vt: *const zkb_transcript_vtable, transcript_repr: *const u64, instances: *const *const u64,
                               lens: *const u32, out: *mut *mut zkb_session) -> i32;
+    pub fn zkb_prove_begin_multi(pk: *mut zkb_pk, kind: i32, vt: *const zkb_transcript_vtable, transcript_repr: *const u64, num_circuits: u32,
+                                 instances: *const *const u64, lens: *const u32, out: *mut *mut zkb_session) -> i32;
     pub fn zkb_prove_advice_phase(s: *mut zkb_session, phase: u32, advice: *const *const u64, challenges_out: *mut u64) -> i32;
     pub fn zkb_prove_finish(s: *mut zkb_session, z_blinds: *const u64, phi_blinds: *const u64, random_poly: *const u64, proof_out: *mut u8,
                             cap: u64, len: *mut u64) -> i32;

@@ -74,7 +74,7 @@ void block_free(zkb_ctx *ctx, void *p, size_t bytes) {
 using namespace zkb;
 
 extern "C" const char *zkb_last_error(void) { return g_err; }
-extern "C" uint32_t zkb_version(void) { return (1u << 16) | 1u; }
+extern "C" uint32_t zkb_version(void) { return (1u << 16) | 2u; }
 
 extern "C" int32_t zkb_init(int32_t device, zkb_ctx **out) {
     ZKB_ARG(out != nullptr);

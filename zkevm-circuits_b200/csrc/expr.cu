@@ -40,6 +40,36 @@ struct RegFile {
     }
 };
 
+// one instruction for the thread owning `row`; `cols` is the slot table the program reads (one circuit's table in a batched launch)
+template <int NREGS, int THREADS, bool SMEM>
+__device__ __forceinline__ void expr_step(const ExprLaunch &L, const Instr in, const Fr *const *cols, uint32_t row, uint32_t mask,
+                                          RegFile<NREGS, THREADS, SMEM> &regs, Fr &acc, Fr &acc2) {
+    switch (in.op) {
+    case OP_LOADCOL: {
+        const int32_t rot = (int32_t)(int16_t)(in.imm >> 16);
+        const uint32_t r = (row + (uint32_t)rot) & mask;
+        regs.set(in.dst, fp_load(cols[in.imm & 0xffffu] + r));
+    } break;
+    case OP_LOADCONST: regs.set(in.dst, fp_load(L.consts + in.imm)); break;
+    case OP_ADD: { Fr a = regs.get(in.a), b = regs.get(in.b); regs.set(in.dst, fp_add(a, b)); } break;
+    case OP_SUB: { Fr a = regs.get(in.a), b = regs.get(in.b); regs.set(in.dst, fp_sub(a, b)); } break;
+    case OP_MUL: { Fr a = regs.get(in.a), b = regs.get(in.b); regs.set(in.dst, fp_mul(a, b)); } break;
+    case OP_NEG: { Fr a = regs.get(in.a); regs.set(in.dst, fp_neg(a)); } break;
+    case OP_HORNER: acc = fp_add(fp_mul(acc, fp_load(L.consts + in.imm)), regs.get(in.a)); break;
+    case OP_STORE: fp_store(L.outs[in.imm] + (size_t)row * L.out_stride + L.out_offset, regs.get(in.a)); break;
+    case OP_STOREACC:
+        fp_store(L.outs[in.imm & 0xffu] + (size_t)row * L.out_stride + L.out_offset, fp_mul(acc, fp_load(L.consts + (in.imm >> 8))));
+        break;
+    case OP_CLEARACC: acc = Fr::zero(); break;
+    case OP_HORNER2: acc2 = fp_add(fp_mul(acc2, fp_load(L.consts + in.imm)), regs.get(in.a)); break;
+    case OP_FOLD:
+        acc = fp_add(fp_mul(acc, fp_load(L.consts + in.imm)), fp_mul(regs.get(in.a), acc2));
+        acc2 = Fr::zero();
+        break;
+    default: break;
+    }
+}
+
 template <int NREGS, int THREADS, bool SMEM>
 __global__ void __launch_bounds__(THREADS) expr_kernel(ExprLaunch L) {
     extern __shared__ uint4 expr_smem[];
@@ -48,55 +78,52 @@ __global__ void __launch_bounds__(THREADS) expr_kernel(ExprLaunch L) {
     if (row >= n) return;
     RegFile<NREGS, THREADS, SMEM> regs(expr_smem);
     Fr acc = Fr::zero(), acc2 = Fr::zero();
-    for (uint32_t pc = 0; pc < L.ncode; ++pc) {
-        const Instr in = L.code[pc];
-        switch (in.op) {
-        case OP_LOADCOL: {
-            const int32_t rot = (int32_t)(int16_t)(in.imm >> 16);
-            const uint32_t r = (row + (uint32_t)rot) & mask;
-            regs.set(in.dst, fp_load(L.cols[in.imm & 0xffffu] + r));
-        } break;
-        case OP_LOADCONST: regs.set(in.dst, fp_load(L.consts + in.imm)); break;
-        case OP_ADD: { Fr a = regs.get(in.a), b = regs.get(in.b); regs.set(in.dst, fp_add(a, b)); } break;
-        case OP_SUB: { Fr a = regs.get(in.a), b = regs.get(in.b); regs.set(in.dst, fp_sub(a, b)); } break;
-        case OP_MUL: { Fr a = regs.get(in.a), b = regs.get(in.b); regs.set(in.dst, fp_mul(a, b)); } break;
-        case OP_NEG: { Fr a = regs.get(in.a); regs.set(in.dst, fp_neg(a)); } break;
-        case OP_HORNER: acc = fp_add(fp_mul(acc, fp_load(L.consts + in.imm)), regs.get(in.a)); break;
-        case OP_STORE: fp_store(L.outs[in.imm] + (size_t)row * L.out_stride + L.out_offset, regs.get(in.a)); break;
-        case OP_STOREACC:
-            fp_store(L.outs[in.imm & 0xffu] + (size_t)row * L.out_stride + L.out_offset, fp_mul(acc, fp_load(L.consts + (in.imm >> 8))));
-            break;
-        case OP_CLEARACC: acc = Fr::zero(); break;
-        case OP_HORNER2: acc2 = fp_add(fp_mul(acc2, fp_load(L.consts + in.imm)), regs.get(in.a)); break;
-        case OP_FOLD:
-            acc = fp_add(fp_mul(acc, fp_load(L.consts + in.imm)), fp_mul(regs.get(in.a), acc2));
-            acc2 = Fr::zero();
-            break;
-        default: break;
-        }
-    }
+    for (uint32_t pc = 0; pc < L.ncode; ++pc) expr_step(L, L.code[pc], L.cols, row, mask, regs, acc, acc2);
 }
 
-template <int NREGS, int THREADS>
-static int32_t launch_smem(const ExprLaunch &L, uint32_t n, cudaStream_t st) {
-    constexpr size_t bytes = (size_t)NREGS * THREADS * 32;
+// Several circuits of one constraint system (create_proof with C circuits): the body code[0, body_len) runs once per circuit,
+// run c reading the slot table at cols + c * stride, and acc / acc2 carry over from one run to the next, so circuit c's
+// constraints continue the Horner chain in y where circuit c - 1 stopped.  The tail code[body_len, ncode) runs once, after the
+// last circuit.  A separate kernel, so the single-circuit launches keep their code.
+struct ExprCircuits {
+    uint32_t count, body_len, stride;
+};
+template <int NREGS, int THREADS, bool SMEM>
+__global__ void __launch_bounds__(THREADS) expr_circuits_kernel(ExprLaunch L, ExprCircuits C) {
+    extern __shared__ uint4 expr_smem[];
+    const uint32_t n = 1u << L.log_n, mask = n - 1;
+    const uint32_t row = blockIdx.x * blockDim.x + threadIdx.x;
+    if (row >= n) return;
+    RegFile<NREGS, THREADS, SMEM> regs(expr_smem);
+    Fr acc = Fr::zero(), acc2 = Fr::zero();
+    for (uint32_t c = 0; c < C.count; ++c) {
+        const Fr *const *cols = L.cols + (size_t)c * C.stride;
+        for (uint32_t pc = 0; pc < C.body_len; ++pc) expr_step(L, L.code[pc], cols, row, mask, regs, acc, acc2);
+    }
+    for (uint32_t pc = C.body_len; pc < L.ncode; ++pc) expr_step(L, L.code[pc], L.cols, row, mask, regs, acc, acc2);
+}
+
+// CIRCUITS: the batched kernel (expr_circuits_kernel, C != nullptr), else expr_kernel
+template <int NREGS, int THREADS, bool SMEM, bool CIRCUITS>
+static int32_t launch(const ExprLaunch &L, const ExprCircuits *C, uint32_t n, cudaStream_t st) {
+    constexpr size_t bytes = SMEM ? (size_t)NREGS * THREADS * 32 : 0;
     static bool attr_set[64] = {};
     int dev = 0;
     cudaGetDevice(&dev);
     if (bytes > 48 * 1024 && dev < 64 && !attr_set[dev]) {
-        ZKB_CUDA(cudaFuncSetAttribute(expr_kernel<NREGS, THREADS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+        if (CIRCUITS) ZKB_CUDA(cudaFuncSetAttribute(expr_circuits_kernel<NREGS, THREADS, SMEM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+        else ZKB_CUDA(cudaFuncSetAttribute(expr_kernel<NREGS, THREADS, SMEM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
         attr_set[dev] = true;
     }
-    expr_kernel<NREGS, THREADS, true><<<(n + THREADS - 1) / THREADS, THREADS, bytes, st>>>(L);
+    const unsigned blocks = (n + THREADS - 1) / THREADS;
+    if (CIRCUITS) expr_circuits_kernel<NREGS, THREADS, SMEM><<<blocks, THREADS, bytes, st>>>(L, *C);
+    else expr_kernel<NREGS, THREADS, SMEM><<<blocks, THREADS, bytes, st>>>(L);
     return ZKB_OK;
 }
 
-// d_code / d_cols / d_consts / d_outs are device pointers
-int32_t expr_run_device(zkb_ctx *ctx, const Instr *d_code, uint32_t ncode, int nregs, const Fr *const *d_cols, const Fr *d_consts,
-                        Fr *const *d_outs, uint32_t log_n, uint32_t out_stride, uint32_t out_offset, cudaStream_t st) {
-    ExprLaunch L{d_code, ncode, d_cols, d_consts, d_outs, log_n, out_stride, out_offset};
-    const uint32_t n = 1u << log_n;
-    const unsigned blocks = (n + 127) / 128;
+template <bool CIRCUITS>
+static int32_t expr_launch(zkb_ctx *ctx, const ExprLaunch &L, const ExprCircuits *C, int nregs, cudaStream_t st) {
+    const uint32_t n = 1u << L.log_n;
     ProfScope ps_(ctx, PROF_EXPR, st);
     // Register file placement, measured on the k = 20 quotient (profiles/r02_expr_kernel_k20_ncu.txt, _smem_ncu.txt):
     //   local memory, 16 registers : 65 ms per coset part, 107 GB of DRAM traffic (registers and columns evict each other from L2), pipe 75 %
@@ -105,13 +132,29 @@ int32_t expr_run_device(zkb_ctx *ctx, const Instr *d_code, uint32_t ncode, int n
     // so programs of <= 8 registers (32 KB per block, 7 blocks per SM) run from shared memory, larger ones from local memory unless
     // ZKB_EXPR_SMEM_REGS=1 asks for the low-traffic variant; the hybrid (8 registers in shared memory, the rest local) is the next step.
     static const bool smem_regs = getenv("ZKB_EXPR_SMEM_REGS") && getenv("ZKB_EXPR_SMEM_REGS")[0] == '1';
-    if (nregs <= 8) ZKB_TRY((launch_smem<8, 128>(L, n, st)));
-    else if (nregs <= 16 && smem_regs) ZKB_TRY((launch_smem<16, 128>(L, n, st)));
-    else if (nregs <= 16) expr_kernel<16, 128, false><<<blocks, 128, 0, st>>>(L);
-    else expr_kernel<64, 128, false><<<blocks, 128, 0, st>>>(L);
+    if (nregs <= 8) ZKB_TRY((launch<8, 128, true, CIRCUITS>(L, C, n, st)));
+    else if (nregs <= 16 && smem_regs) ZKB_TRY((launch<16, 128, true, CIRCUITS>(L, C, n, st)));
+    else if (nregs <= 16) ZKB_TRY((launch<16, 128, false, CIRCUITS>(L, C, n, st)));
+    else ZKB_TRY((launch<64, 128, false, CIRCUITS>(L, C, n, st)));
     ctx->launches++;
     ZKB_CUDA(cudaGetLastError());
     return ZKB_OK;
+}
+
+// d_code / d_cols / d_consts / d_outs are device pointers
+int32_t expr_run_device(zkb_ctx *ctx, const Instr *d_code, uint32_t ncode, int nregs, const Fr *const *d_cols, const Fr *d_consts,
+                        Fr *const *d_outs, uint32_t log_n, uint32_t out_stride, uint32_t out_offset, cudaStream_t st) {
+    const ExprLaunch L{d_code, ncode, d_cols, d_consts, d_outs, log_n, out_stride, out_offset};
+    return expr_launch<false>(ctx, L, nullptr, nregs, st);
+}
+// the same program over `count` circuits: d_cols holds count slot tables of `stride` slots; code[0, body_len) runs per circuit,
+// code[body_len, ncode) once at the end (expr_circuits_kernel)
+int32_t expr_run_circuits_device(zkb_ctx *ctx, const Instr *d_code, uint32_t ncode, uint32_t body_len, int nregs, const Fr *const *d_cols,
+                                 uint32_t count, uint32_t stride, const Fr *d_consts, Fr *const *d_outs, uint32_t log_n, uint32_t out_stride,
+                                 uint32_t out_offset, cudaStream_t st) {
+    const ExprLaunch L{d_code, ncode, d_cols, d_consts, d_outs, log_n, out_stride, out_offset};
+    const ExprCircuits C{count, body_len, stride};
+    return expr_launch<true>(ctx, L, &C, nregs, st);
 }
 
 }  // namespace zkb

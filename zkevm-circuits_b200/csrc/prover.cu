@@ -31,6 +31,9 @@ namespace zkb {
 
 int32_t expr_run_device(zkb_ctx *ctx, const Instr *d_code, uint32_t ncode, int nregs, const Fr *const *d_cols, const Fr *d_consts,
                         Fr *const *d_outs, uint32_t log_n, uint32_t out_stride, uint32_t out_offset, cudaStream_t st);
+int32_t expr_run_circuits_device(zkb_ctx *ctx, const Instr *d_code, uint32_t ncode, uint32_t body_len, int nregs, const Fr *const *d_cols,
+                                 uint32_t count, uint32_t stride, const Fr *d_consts, Fr *const *d_outs, uint32_t log_n, uint32_t out_stride,
+                                 uint32_t out_offset, cudaStream_t st);
 
 // ---------------------------------------------------------------------------------------------------------- CSF
 enum { N_CONST = 0, N_FIXED = 1, N_ADVICE = 2, N_INSTANCE = 3, N_CHALLENGE = 4, N_NEG = 5, N_ADD = 6, N_MUL = 7, N_SCALED = 8 };
@@ -339,12 +342,16 @@ struct zkb_pk {
     }
 };
 
+// One proof of `nc` circuits of the same constraint system (create_proof's `circuits: &[C]`).  Per-circuit columns are
+// circuit-major: circuit c's instance column i is inst_values[c * ni + i], its advice column j is adv_values[c * na + j].
 struct zkb_session {
     zkb_pk *pk = nullptr;
+    uint32_t nc = 1;
     Transcript tr;
     DevPool pool;
     std::vector<Fr *> inst_values, inst_polys, adv_values;
-    // columns handed over ahead of their phase (zkb_prove_upload_advice): staged device copies, consumed by zkb_prove_advice_phase
+    // columns handed over ahead of their phase (zkb_prove_upload_advice), keyed by c * na + column: staged device copies, consumed
+    // by zkb_prove_advice_phase
     std::map<uint32_t, Fr *> early_cols;
     std::vector<Fr> challenges;
     uint32_t next_phase = 0;
@@ -857,23 +864,33 @@ extern "C" int32_t zkb_prove_begin(zkb_pk *pk, const uint64_t transcript_repr[4]
     return zkb_prove_begin_ex(pk, 0, transcript_repr, instance_values, instance_lens, out);
 }
 static int32_t prove_begin_common(zkb_pk *pk, int32_t transcript_kind, const zkb_transcript_vtable *vt, const uint64_t transcript_repr[4],
-                                  const uint64_t *const *instance_values, const uint32_t *instance_lens, zkb_session **out);
+                                  uint32_t num_circuits, const uint64_t *const *instance_values, const uint32_t *instance_lens, zkb_session **out);
 extern "C" int32_t zkb_prove_begin_ex(zkb_pk *pk, int32_t transcript_kind, const uint64_t transcript_repr[4], const uint64_t *const *instance_values,
                                       const uint32_t *instance_lens, zkb_session **out) {
     ZKB_ARG(transcript_kind >= TR_BLAKE2B && transcript_kind <= TR_EVM);
-    return prove_begin_common(pk, transcript_kind, nullptr, transcript_repr, instance_values, instance_lens, out);
+    return prove_begin_common(pk, transcript_kind, nullptr, transcript_repr, 1, instance_values, instance_lens, out);
 }
 extern "C" int32_t zkb_prove_begin_cb(zkb_pk *pk, const zkb_transcript_vtable *vt, const uint64_t transcript_repr[4],
                                       const uint64_t *const *instance_values, const uint32_t *instance_lens, zkb_session **out) {
     ZKB_ARG(vt && vt->common_scalar && vt->write_scalar && vt->write_point && vt->squeeze_challenge);
-    return prove_begin_common(pk, TR_CALLER, vt, transcript_repr, instance_values, instance_lens, out);
+    return prove_begin_common(pk, TR_CALLER, vt, transcript_repr, 1, instance_values, instance_lens, out);
+}
+extern "C" int32_t zkb_prove_begin_multi(zkb_pk *pk, int32_t transcript_kind, const zkb_transcript_vtable *vt, const uint64_t transcript_repr[4],
+                                         uint32_t num_circuits, const uint64_t *const *instance_values, const uint32_t *instance_lens,
+                                         zkb_session **out) {
+    ZKB_ARG(transcript_kind >= TR_BLAKE2B && transcript_kind <= TR_CALLER && num_circuits >= 1);
+    if (transcript_kind == TR_CALLER) ZKB_ARG(vt && vt->common_scalar && vt->write_scalar && vt->write_point && vt->squeeze_challenge);
+    else ZKB_ARG(vt == nullptr);
+    return prove_begin_common(pk, transcript_kind, vt, transcript_repr, num_circuits, instance_values, instance_lens, out);
 }
 static int32_t prove_begin_common(zkb_pk *pk, int32_t transcript_kind, const zkb_transcript_vtable *vt, const uint64_t transcript_repr[4],
-                                  const uint64_t *const *instance_values, const uint32_t *instance_lens, zkb_session **out) {
+                                  uint32_t num_circuits, const uint64_t *const *instance_values, const uint32_t *instance_lens, zkb_session **out) {
     ZKB_ARG(pk && transcript_repr && out && (pk->cs.ni == 0 || (instance_values && instance_lens)));
+    ZKB_ARG((uint64_t)num_circuits * (pk->cs.na + pk->cs.ni + pk->cs.lookups.size() + pk->nsets) < (1ull << 31));
     ZKB_CUDA(cudaSetDevice(pk->ctx->device));
     std::unique_ptr<zkb_session> s(new zkb_session());
     s->pk = pk;
+    s->nc = num_circuits;
     s->tr.kind = (TranscriptKind)transcript_kind;
     if (vt) s->tr.vt = *vt;
     s->pool.ctx = pk->ctx;
@@ -883,9 +900,11 @@ static int32_t prove_begin_common(zkb_pk *pk, int32_t transcript_kind, const zkb
     Fr repr;
     memcpy(repr.l, transcript_repr, 32);
     s->tr.common_scalar(repr);  // vk.hash_into(transcript)
-    s->inst_values.resize(cs.ni);
-    s->inst_polys.resize(cs.ni);
-    for (uint32_t c = 0; c < cs.ni; ++c) {
+    // instance values circuit-major: for each circuit, for each instance column, every value
+    const uint32_t ninst = num_circuits * cs.ni;
+    s->inst_values.resize(ninst);
+    s->inst_polys.resize(ninst);
+    for (uint32_t c = 0; c < ninst; ++c) {
         ZKB_ARG(instance_lens[c] <= n - (cs.bf + 1));
         ZKB_TRY(s->pool.fr(n, &s->inst_values[c]));
         ZKB_TRY(s->pool.fr(n, &s->inst_polys[c]));
@@ -898,7 +917,7 @@ static int32_t prove_begin_common(zkb_pk *pk, int32_t transcript_kind, const zkb
         if (instance_lens[c]) ZKB_CUDA(cudaMemcpyAsync(s->inst_values[c], instance_values[c], (size_t)instance_lens[c] * sizeof(Fr), cudaMemcpyHostToDevice, st));
         ZKB_TRY(lagrange_to_coeff(pk, s->inst_values[c], s->inst_polys[c], st));
     }
-    s->adv_values.assign(cs.na, nullptr);
+    s->adv_values.assign((size_t)num_circuits * cs.na, nullptr);
     s->challenges.assign(cs.nch, Fr::zero());
     ZKB_CUDA(cudaStreamSynchronize(st));
     ZKB_TRY(s->tr.status());
@@ -909,10 +928,11 @@ static int32_t prove_begin_common(zkb_pk *pk, int32_t transcript_kind, const zkb
 // Witness-side overlap (SURVEY 8f row 4): `synthesize` assigns sub-circuit after sub-circuit (super_circuit.rs:714-806), so the columns
 // of a phase become final one at a time.  The shim may hand each finished column over immediately: the copy runs on the copy stream
 // while Rust keeps synthesising, and zkb_prove_advice_phase later finds the column already in HBM (its pointer may then be NULL).
+// In a session of C circuits `column` is c * num_advice + the column of circuit c.
 extern "C" int32_t zkb_prove_upload_advice(zkb_session *s, uint32_t column, const uint64_t *values) {
-    ZKB_ARG(s && values && column < s->pk->cs.na);
+    ZKB_ARG(s && values && (uint64_t)column < (uint64_t)s->nc * s->pk->cs.na);
     zkb_pk *pk = s->pk;
-    if (s->finished || pk->cs.adv_phase[column] < s->next_phase) { set_error("column %u belongs to a phase that is already committed", column); return ZKB_ERR_STATE; }
+    if (s->finished || pk->cs.adv_phase[column % pk->cs.na] < s->next_phase) { set_error("column %u belongs to a phase that is already committed", column); return ZKB_ERR_STATE; }
     ZKB_CUDA(cudaSetDevice(pk->ctx->device));
     Fr *&d = s->early_cols[column];
     if (!d) ZKB_TRY(s->pool.fr(pk->n, &d));
@@ -931,13 +951,18 @@ extern "C" int32_t zkb_prove_advice_phase(zkb_session *s, uint32_t phase, const 
     // H2D on the copy stream, batch by batch; the MSM of batch b waits only for batch b's event, so the copies of the
     // following batches overlap it (pinned caller buffers; pageable ones are staged synchronously by the driver anyway).
     // Multi-GPU: a rank uploads and commits only the columns it owns, then the column data is gathered over NVLink.
+    // circuit-major: circuit 0's columns of this phase, then circuit 1's, ... (the order of the commitments in the transcript)
     std::vector<const uint64_t *> phase_src;
     std::vector<uint32_t> phase_idx;
-    for (uint32_t c = 0; c < cs.na; ++c) {
-        if (cs.adv_phase[c] != phase) continue;
+    for (uint32_t c = 0; c < s->nc * cs.na; ++c) {
+        if (cs.adv_phase[c % cs.na] != phase) continue;
         auto early = s->early_cols.find(c);
         const uint64_t *src = advice_columns[c] ? advice_columns[c] : (early != s->early_cols.end() ? (const uint64_t *)early->second : nullptr);
-        if (!src) { set_error("advice column %u of phase %u was neither passed nor uploaded ahead", c, phase); return ZKB_ERR_ARG; }
+        if (!src) {
+            if (s->nc == 1) set_error("advice column %u of phase %u was neither passed nor uploaded ahead", c, phase);
+            else set_error("advice column %u of circuit %u (phase %u) was neither passed nor uploaded ahead", c % cs.na, c / cs.na, phase);
+            return ZKB_ERR_ARG;
+        }
         phase_src.push_back(src);   // a staged copy is a device pointer: the gather into the phase slab below is then device-to-device
         phase_idx.push_back(c);
     }
@@ -1033,27 +1058,33 @@ struct RotationSet {
     std::vector<std::vector<Fr>> r_coeffs;     // per commitment: low-degree interpolant through (pts, evaluations)
 };
 
-// What the stages of one create_proof hand to each other; lives for one call of prove_finish_impl.
+// What the stages of one create_proof hand to each other; lives for one call of prove_finish_impl.  With C circuits every
+// per-circuit vector (lookups, permutation sets, their polynomials) is circuit-major: unit u belongs to circuit u / count.
 struct ProofState {
     zkb_session *s;
     zkb_pk *pk;
     zkb_ctx *ctx;
     const Csf &cs;
     uint64_t n;
-    uint32_t k, bf;
+    uint32_t k, bf, nc;
     cudaStream_t st;
     DevPool &pool;
-    Deal lk_deal;   // multi-GPU: the lookup arguments are dealt, prepared and summed by the rank that owns them
+    Deal lk_deal;   // multi-GPU: the lookup arguments of all circuits are dealt, prepared and summed by the rank that owns them
     Fr theta, beta, gamma, y, x, sy, sv, su;   // sy, sv, su: SHPLONK's y, v, u
-    Fr **d_vcols = nullptr;   // value-domain column table: [fixed | advice | instance | sigma | omega_pows]
+    // value-domain column tables, one per circuit (circuit c's at d_vcols + c * vstride): [fixed | advice | instance | sigma | omega_pows]
+    Fr **d_vcols = nullptr;
+    uint32_t vstride = 0;
     std::vector<std::vector<Fr *>> lk_f;      // compressed inputs per lookup / input set
     std::vector<Fr *> lk_t, lk_m, zs, phis;   // compressed tables, multiplicities, permutation grand products, lookup grand sums
     Fr *random_poly = nullptr;
     std::vector<Fr *> adv_polys, z_polys, phi_polys, m_polys;   // coefficient forms
-    // quotient: coset-domain slot table [fixed | advice | instance | sigma | z | phi | m | l0 | l_last | l_blind | X]; the program
-    // (common body + one trailing STOREACC slot rewritten per coset part); h on the extended domain, then its d - 1 pieces
+    // quotient: coset-domain slot table of one circuit [fixed | advice | instance | sigma | z | phi | m | l0 | l_last | l_blind | X]
+    // (q_stride slots; C circuits: C tables, the shared slots repeat); qpolys holds every distinct polynomial once, q_slot maps each
+    // table entry to it; the program (common body + one trailing STOREACC slot rewritten per coset part); h on the extended
+    // domain, then its d - 1 pieces
     std::vector<Fr *> qpolys;
-    uint32_t q_sigma0 = 0, q_z0 = 0, q_phi0 = 0, q_m0 = 0, q_l0 = 0;
+    std::vector<uint32_t> q_slot;
+    uint32_t q_sigma0 = 0, q_z0 = 0, q_phi0 = 0, q_m0 = 0, q_l0 = 0, q_stride = 0;
     DeviceProgram qdp;
     size_t q_base_len = 0;
     std::vector<uint32_t> tinv_idx;
@@ -1069,8 +1100,8 @@ struct ProofState {
     Fr *hx = nullptr, *work = nullptr, *work2 = nullptr, *d_small = nullptr;
 
     explicit ProofState(zkb_session *sess)
-        : s(sess), pk(sess->pk), ctx(pk->ctx), cs(pk->cs), n(pk->n), k(pk->cs.k), bf(pk->cs.bf), st(pk->ctx->stream), pool(sess->pool),
-          lk_deal(pk->ctx, pk->cs.lookups.size()) {}
+        : s(sess), pk(sess->pk), ctx(pk->ctx), cs(pk->cs), n(pk->n), k(pk->cs.k), bf(pk->cs.bf), nc(sess->nc), st(pk->ctx->stream), pool(sess->pool),
+          lk_deal(pk->ctx, (size_t)sess->nc * pk->cs.lookups.size()) {}
 };
 
 // mv_lookup/prover.rs::prepare: compress inputs and table with theta, multiplicities m over the usable rows, commit m
@@ -1079,31 +1110,35 @@ static int32_t lookups_prepare(ProofState &p) {
     const Csf &cs = p.cs;
     const uint64_t n = p.n;
     const uint32_t usable = (uint32_t)(n - p.bf - 1);
-    const size_t nl = cs.lookups.size();
+    const size_t nl = cs.lookups.size(), nu = p.nc * nl;   // nu: lookup arguments of all circuits
     cudaStream_t st = p.st;
     DevPool &pool = p.pool;
     const SlotMap vsm{0, cs.nf, cs.nf + cs.na};
     std::vector<Fr *> vcols;
-    for (auto q : p.pk->fixed_values) vcols.push_back(q);
-    for (auto q : s->adv_values) vcols.push_back(q);
-    for (auto q : s->inst_values) vcols.push_back(q);
-    for (auto q : p.pk->sigma_values) vcols.push_back(q);
-    vcols.push_back(p.pk->omega_pows);
+    for (uint32_t c = 0; c < p.nc; ++c) {
+        for (auto q : p.pk->fixed_values) vcols.push_back(q);
+        for (uint32_t i = 0; i < cs.na; ++i) vcols.push_back(s->adv_values[(size_t)c * cs.na + i]);
+        for (uint32_t i = 0; i < cs.ni; ++i) vcols.push_back(s->inst_values[(size_t)c * cs.ni + i]);
+        for (auto q : p.pk->sigma_values) vcols.push_back(q);
+        vcols.push_back(p.pk->omega_pows);
+    }
+    p.vstride = (uint32_t)(vcols.size() / p.nc);
     ZKB_TRY(upload_table(pool, vcols, &p.d_vcols, st));
 
-    p.lk_f.resize(nl);
-    p.lk_t.resize(nl);
-    p.lk_m.resize(nl);
+    p.lk_f.resize(nu);
+    p.lk_t.resize(nu);
+    p.lk_m.resize(nu);
     // m columns live in one slab, completed by one all-gather when dealt
     const Deal &deal = p.lk_deal;
     Fr *m_slab = nullptr;
-    if (nl) {
+    if (nu) {
         ZKB_TRY(pool.fr(deal.padded() * n, &m_slab));
-        for (size_t l = 0; l < nl; ++l) p.lk_m[l] = m_slab + l * n;
+        for (size_t u = 0; u < nu; ++u) p.lk_m[u] = m_slab + u * n;
     }
     uint64_t lookup_errors = 0;
-    for (size_t l = 0; l < nl; ++l) {
-        if (!deal.mine(l)) continue;
+    for (size_t u = 0; u < nu; ++u) {
+        if (!deal.mine(u)) continue;
+        const size_t c = u / nl, l = u % nl;
         const CsfLookup &lk = cs.lookups[l];
         ExprBuilder eb;
         ProgramBuilder pb(eb);
@@ -1113,15 +1148,15 @@ static int32_t lookups_prepare(ProofState &p) {
         for (size_t j = 0; j < lk.inputs.size(); ++j) {
             Fr *a;
             ZKB_TRY(pool.fr(n, &a));
-            p.lk_f[l].push_back(a);
+            p.lk_f[u].push_back(a);
             outs.push_back(a);
             roots.push_back({compress_exprs(cs, lk.inputs[j], eb, vsm, s->challenges, memo, p.theta), ProgramBuilder::STORE, (uint32_t)j});
         }
-        ZKB_TRY(pool.fr(n, &p.lk_t[l]));
-        outs.push_back(p.lk_t[l]);
+        ZKB_TRY(pool.fr(n, &p.lk_t[u]));
+        outs.push_back(p.lk_t[u]);
         roots.push_back({compress_exprs(cs, lk.table, eb, vsm, s->challenges, memo, p.theta), ProgramBuilder::STORE, (uint32_t)lk.inputs.size()});
         if (!pb.scope(roots)) { set_error("lookup %zu: %s", l, pb.error.c_str()); return ZKB_ERR_ARG; }
-        ZKB_TRY(run_program(s, pb, eb, p.d_vcols, outs, st));
+        ZKB_TRY(run_program(s, pb, eb, p.d_vcols + c * p.vstride, outs, st));
         // multiplicities over the usable rows
         uint32_t tsize = 1;
         while (tsize < 2 * usable) tsize <<= 1;
@@ -1133,15 +1168,16 @@ static int32_t lookups_prepare(ProofState &p) {
         ZKB_CUDA(cudaMemsetAsync(slots, 0, (size_t)tsize * 4, st));
         ZKB_CUDA(cudaMemsetAsync(counts, 0, (size_t)n * 4 + 16, st));
         const unsigned ub = (usable + 255) / 256;
-        m_insert_kernel<<<ub, 256, 0, st>>>(p.lk_t[l], usable, slots, tsize - 1);
-        for (size_t j = 0; j < lk.inputs.size(); ++j) m_count_kernel<<<ub, 256, 0, st>>>(p.lk_f[l][j], p.lk_t[l], usable, slots, tsize - 1, counts, d_err);
-        counts_to_fr_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(counts, (uint32_t)n, p.lk_m[l]);
+        m_insert_kernel<<<ub, 256, 0, st>>>(p.lk_t[u], usable, slots, tsize - 1);
+        for (size_t j = 0; j < lk.inputs.size(); ++j) m_count_kernel<<<ub, 256, 0, st>>>(p.lk_f[u][j], p.lk_t[u], usable, slots, tsize - 1, counts, d_err);
+        counts_to_fr_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(counts, (uint32_t)n, p.lk_m[u]);
         p.ctx->launches += 2 + lk.inputs.size();
         int herr = 0;
         ZKB_CUDA(cudaMemcpyAsync(&herr, d_err, 4, cudaMemcpyDeviceToHost, st));
         ZKB_CUDA(cudaStreamSynchronize(st));
         if (herr) {
-            set_error("lookup %zu: an input row is not in the table (unsatisfied witness)", l);
+            if (p.nc == 1) set_error("lookup %zu: an input row is not in the table (unsatisfied witness)", l);
+            else set_error("circuit %zu, lookup %zu: an input row is not in the table (unsatisfied witness)", c, l);
             if (!deal.on) return ZKB_ERR_ARG;
             lookup_errors++;   // multi-GPU: every rank must learn about it before anyone leaves the collective sequence
         }
@@ -1175,22 +1211,26 @@ static int32_t permutation_commit(ProofState &p, const uint64_t *z_blinds) {
     const SlotMap vsm{0, cs.nf, cs.nf + cs.na};
     const uint32_t v_sigma0 = cs.nf + cs.na + cs.ni, v_omega = v_sigma0 + (uint32_t)cs.perm.size();
     const Fr delta = perm_delta();
-    // Multi-GPU: the sets are dealt.  Upstream chains them (z_i[0] = last value of z_{i-1}), which is sequential; here every set is
-    // scanned from 1 and rescaled afterwards by c_i = product of the previous sets' last values -- the same field elements
-    // (z_i = c_i * z'_i row by row), with only the nsets last values crossing the ranks before the columns are gathered.
-    const Deal dp_sets(ctx, pk->nsets);
-    p.zs.resize(pk->nsets);
+    // Multi-GPU: the sets of all circuits are dealt.  Upstream chains a circuit's sets (z_i[0] = last value of z_{i-1}; every
+    // circuit's first set starts at 1), which is sequential; here every set is scanned from 1 and rescaled afterwards by c_i = product
+    // of the same circuit's previous sets' last values -- the same field elements (z_i = c_i * z'_i row by row), with only the last
+    // values crossing the ranks before the columns are gathered.
+    const uint32_t nsets = pk->nsets, nu = p.nc * nsets;   // unit u = set u % nsets of circuit u / nsets
+    const Deal dp_sets(ctx, nu);
+    p.zs.resize(nu);
     Fr *z_slab = nullptr;
     ZKB_TRY(p.pool.fr(std::max<size_t>(1, dp_sets.padded()) * n, &z_slab));
-    for (uint32_t si = 0; si < pk->nsets; ++si) p.zs[si] = z_slab + (size_t)si * n;
+    for (uint32_t u = 0; u < nu; ++u) p.zs[u] = z_slab + (size_t)u * n;
     Fr *num, *den, *tmp;
     ZKB_TRY(p.pool.fr(n, &num));
     ZKB_TRY(p.pool.fr(n, &den));
     ZKB_TRY(p.pool.fr(n, &tmp));
     std::vector<Fr> lasts(std::max<size_t>(1, dp_sets.padded()), one);
     Fr last_z = one;
-    for (uint32_t si = 0; si < pk->nsets; ++si) {
-        if (!dp_sets.mine(si)) continue;
+    for (uint32_t u = 0; u < nu; ++u) {
+        const uint32_t c = u / nsets, si = u % nsets;
+        if (si == 0) last_z = one;
+        if (!dp_sets.mine(u)) continue;
         ExprBuilder eb;
         ProgramBuilder pb(eb);
         uint32_t nnum = 0, nden = 0;
@@ -1206,26 +1246,27 @@ static int32_t permutation_commit(ProofState &p, const uint64_t *z_blinds) {
             delta_pow = fp_mul(delta_pow, delta);
         }
         if (!pb.scope({{nnum, ProgramBuilder::STORE, 0}, {nden, ProgramBuilder::STORE, 1}})) { set_error("permutation: %s", pb.error.c_str()); return ZKB_ERR_ARG; }
-        ZKB_TRY(run_program(p.s, pb, eb, p.d_vcols, {num, den}, st));
+        ZKB_TRY(run_program(p.s, pb, eb, p.d_vcols + (size_t)c * p.vstride, {num, den}, st));
         ZKB_TRY(batch_invert_device(ctx, den, tmp, n, st));
         mul_arrays_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(num, tmp, den, n);  // den <- modified values
         ctx->launches++;
         // one GPU: chained exactly like upstream (init = previous last value); dealt: from 1, rescaled below
-        ZKB_TRY(prefix_product_device(ctx, den, n, dp_sets.on ? one : last_z, p.zs[si], st));
-        ZKB_CUDA(cudaMemcpyAsync(&last_z, p.zs[si] + (n - bf - 1), sizeof(Fr), cudaMemcpyDeviceToHost, st));
+        ZKB_TRY(prefix_product_device(ctx, den, n, dp_sets.on ? one : last_z, p.zs[u], st));
+        ZKB_CUDA(cudaMemcpyAsync(&last_z, p.zs[u] + (n - bf - 1), sizeof(Fr), cudaMemcpyDeviceToHost, st));
         ZKB_CUDA(cudaStreamSynchronize(st));
-        lasts[si] = last_z;
-        if (!dp_sets.on) ZKB_CUDA(cudaMemcpyAsync(p.zs[si] + (n - bf), z_blinds + 4ull * bf * si, (size_t)bf * sizeof(Fr), cudaMemcpyHostToDevice, st));
+        lasts[u] = last_z;
+        if (!dp_sets.on) ZKB_CUDA(cudaMemcpyAsync(p.zs[u] + (n - bf), z_blinds + 4ull * bf * u, (size_t)bf * sizeof(Fr), cudaMemcpyHostToDevice, st));
     }
     if (dp_sets.on) {
         ZKB_TRY(deal_gather_host(ctx, dp_sets, lasts.data(), sizeof(Fr), st));
-        Fr c = one;   // c_i = prod_{j < i} last'_j
-        for (uint32_t si = 0; si < pk->nsets; ++si) {
-            if (dp_sets.mine(si)) {
-                if (!(c == one)) { scale_const_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(p.zs[si], c, n); ctx->launches++; }
-                ZKB_CUDA(cudaMemcpyAsync(p.zs[si] + (n - bf), z_blinds + 4ull * bf * si, (size_t)bf * sizeof(Fr), cudaMemcpyHostToDevice, st));
+        Fr c = one;   // c_i = prod_{j < i} last'_j over the sets of the same circuit
+        for (uint32_t u = 0; u < nu; ++u) {
+            if (u % nsets == 0) c = one;
+            if (dp_sets.mine(u)) {
+                if (!(c == one)) { scale_const_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(p.zs[u], c, n); ctx->launches++; }
+                ZKB_CUDA(cudaMemcpyAsync(p.zs[u] + (n - bf), z_blinds + 4ull * bf * u, (size_t)bf * sizeof(Fr), cudaMemcpyHostToDevice, st));
             }
-            c = fp_mul(c, lasts[si]);
+            c = fp_mul(c, lasts[u]);
         }
         ZKB_TRY(deal_gather(ctx, dp_sets, z_slab, n * sizeof(Fr), st));
     }
@@ -1235,7 +1276,7 @@ static int32_t permutation_commit(ProofState &p, const uint64_t *z_blinds) {
 // mv_lookup/prover.rs::commit_grand_sum: phi = prefix sum of sum_j 1/(f_j + beta) - m/(t + beta) (phi_blinds: bf values per lookup)
 static int32_t lookups_commit_sums(ProofState &p, const uint64_t *phi_blinds) {
     const uint64_t n = p.n;
-    const size_t nl = p.cs.lookups.size();
+    const size_t nl = p.lk_m.size();   // lookup arguments of all circuits, circuit-major
     cudaStream_t st = p.st;
     DevPool &pool = p.pool;
     p.phis.resize(nl);
@@ -1326,27 +1367,46 @@ static int32_t to_coefficients(ProofState &p) {
 }
 
 // evaluation.rs::evaluate_h: the quotient numerator as ONE interpreter program over the coset-domain slot table, every constraint
-// folded in with Horner in y, in upstream's order (gates, permutation, lookups)
+// folded in with Horner in y, in upstream's order (gates, permutation, lookups).  With C circuits upstream loops over the circuits
+// and keeps folding into the same accumulator; here the kernel runs the same program once per circuit's slot table and carries the
+// accumulator over, so h = sum_c A_c y^(K (C - 1 - c)) for the single-circuit numerators A_c of K folded constraints each.
 static int32_t quotient_program(ProofState &p) {
     zkb_pk *pk = p.pk;
     const Csf &cs = p.cs;
     const std::vector<Fr> &challenges = p.s->challenges;
     const Fr one = Fr::one();
-    auto append = [&](const std::vector<Fr *> &polys) {   // -> first slot of `polys`
-        const uint32_t at = (uint32_t)p.qpolys.size();
-        p.qpolys.insert(p.qpolys.end(), polys.begin(), polys.end());
-        return at;
-    };
-    append(pk->fixed_polys);
-    append(p.adv_polys);
-    append(p.s->inst_polys);
-    p.q_sigma0 = append(pk->sigma_polys);
-    p.q_z0 = append(p.z_polys);
-    p.q_phi0 = append(p.phi_polys);
-    p.q_m0 = append(p.m_polys);
-    p.q_l0 = append({pk->l0_poly, pk->llast_poly, pk->lblind_poly, pk->xid_poly});
+    const uint32_t ns = pk->nsets, nl = (uint32_t)cs.lookups.size();
+    p.q_sigma0 = cs.nf + cs.na + cs.ni;
+    p.q_z0 = p.q_sigma0 + (uint32_t)cs.perm.size();
+    p.q_phi0 = p.q_z0 + ns;
+    p.q_m0 = p.q_phi0 + nl;
+    p.q_l0 = p.q_m0 + nl;
+    p.q_stride = p.q_l0 + 4;
     const uint32_t q_l0 = p.q_l0, q_llast = q_l0 + 1, q_lblind = q_l0 + 2, q_x = q_l0 + 3;
-    ZKB_ARG(p.qpolys.size() < 65536);
+    ZKB_ARG(p.q_stride < 65536);
+    auto table_of = [&](uint32_t c) {   // the slot table of circuit c (coefficient forms)
+        std::vector<Fr *> t(pk->fixed_polys);
+        auto add = [&](const std::vector<Fr *> &v, size_t first, size_t count) { t.insert(t.end(), v.begin() + first, v.begin() + first + count); };
+        add(p.adv_polys, (size_t)c * cs.na, cs.na);
+        add(p.s->inst_polys, (size_t)c * cs.ni, cs.ni);
+        add(pk->sigma_polys, 0, cs.perm.size());
+        add(p.z_polys, (size_t)c * ns, ns);
+        add(p.phi_polys, (size_t)c * nl, nl);
+        add(p.m_polys, (size_t)c * nl, nl);
+        t.insert(t.end(), {pk->l0_poly, pk->llast_poly, pk->lblind_poly, pk->xid_poly});
+        return t;
+    };
+    auto scoped = [&](uint32_t slot) { return (slot >= cs.nf && slot < p.q_sigma0) || (slot >= p.q_z0 && slot < p.q_l0); };
+    p.qpolys = table_of(0);
+    for (uint32_t i = 0; i < p.q_stride; ++i) p.q_slot.push_back(i);
+    for (uint32_t c = 1; c < p.nc; ++c) {
+        const std::vector<Fr *> t = table_of(c);
+        for (uint32_t i = 0; i < p.q_stride; ++i) {
+            if (!scoped(i)) { p.q_slot.push_back(i); continue; }
+            p.q_slot.push_back((uint32_t)p.qpolys.size());
+            p.qpolys.push_back(t[i]);
+        }
+    }
     const SlotMap qsm{0, cs.nf, cs.nf + cs.na};
 
     ExprBuilder qeb;
@@ -1457,7 +1517,7 @@ static int32_t quotient_evaluate(ProofState &p) {
     cudaStream_t st = p.st;
     DevPool &pool = p.pool;
     const std::vector<Fr *> &qpolys = p.qpolys;
-    Fr *slab, *pows;
+    Fr *slab, *pows;   // slab: coset values of every distinct polynomial of the slot tables
     ZKB_TRY(pool.fr(qpolys.size() * n, &slab));
     ZKB_TRY(pool.fr(n, &pows));
     ZKB_TRY(pool.fr(pk->N, &p.h_ext));
@@ -1476,8 +1536,8 @@ static int32_t quotient_evaluate(ProofState &p) {
     for (size_t i = 0; i < qpolys.size(); ++i) {
         if (cache_idx[i] < 0) { ntt_src.push_back(qpolys[i]); ntt_dst.push_back(qcols[i]); }
     }
-    Fr **d_qcols = nullptr, **d_hout = nullptr;
-    ZKB_TRY(pool.alloc(qcols.size() * sizeof(Fr *) + 8, (void **)&d_qcols));
+    Fr **d_qcols = nullptr, **d_hout = nullptr;   // d_qcols: the slot tables of all circuits
+    ZKB_TRY(pool.alloc(p.q_slot.size() * sizeof(Fr *) + 8, (void **)&d_qcols));
     // multi-GPU: coset parts are dealt in contiguous blocks; a rank writes its parts as contiguous n-element rows of h_parts, the rows
     // are all-gathered and interleaved into the extended-domain order h_ext[j + E i] the inverse transform expects
     const Deal dq(ctx, pk->E);
@@ -1493,12 +1553,16 @@ static int32_t quotient_evaluate(ProofState &p) {
         if (cached)
             for (size_t i = 0; i < qpolys.size(); ++i)
                 if (cache_idx[i] >= 0) cols_j[i] = pk->coset_cache[j][cache_idx[i]];
+        std::vector<Fr *> tables(p.q_slot.size());
+        for (size_t t = 0; t < tables.size(); ++t) tables[t] = cols_j[p.q_slot[t]];
         Instr tail{OP_STOREACC, 0, 0, 0, 0u | (p.tinv_idx[j] << 8)};
-        ZKB_CUDA(cudaMemcpyAsync(d_qcols, cols_j.data(), cols_j.size() * sizeof(Fr *), cudaMemcpyHostToDevice, st));
+        ZKB_CUDA(cudaMemcpyAsync(d_qcols, tables.data(), tables.size() * sizeof(Fr *), cudaMemcpyHostToDevice, st));
         ZKB_CUDA(cudaMemcpyAsync(qdp.code + p.q_base_len, &tail, sizeof(Instr), cudaMemcpyHostToDevice, st));
-        if (dq.on) ZKB_TRY(expr_run_device(ctx, qdp.code, qdp.ncode, qdp.nregs, d_qcols, qdp.consts, d_hout, p.k, 1, (uint32_t)((uint64_t)j * n), st));
-        else ZKB_TRY(expr_run_device(ctx, qdp.code, qdp.ncode, qdp.nregs, d_qcols, qdp.consts, d_hout, p.k, pk->E, j, st));
-        ZKB_CUDA(cudaStreamSynchronize(st));  // `tail` and `cols_j` live on the stack
+        const uint32_t out_stride = dq.on ? 1 : pk->E, out_offset = dq.on ? (uint32_t)((uint64_t)j * n) : j;
+        if (p.nc == 1) ZKB_TRY(expr_run_device(ctx, qdp.code, qdp.ncode, qdp.nregs, d_qcols, qdp.consts, d_hout, p.k, out_stride, out_offset, st));
+        else ZKB_TRY(expr_run_circuits_device(ctx, qdp.code, qdp.ncode, (uint32_t)p.q_base_len, qdp.nregs, d_qcols, p.nc, p.q_stride, qdp.consts, d_hout,
+                                              p.k, out_stride, out_offset, st));
+        ZKB_CUDA(cudaStreamSynchronize(st));  // `tail` and `tables` live on the stack
     }
     if (dq.on) {
         ZKB_TRY(deal_gather(ctx, dq, h_parts, n * sizeof(Fr), st));
@@ -1537,27 +1601,32 @@ static int32_t evaluate(ProofState &p) {
         ZKB_TRY(lincomb(p.s, pieces, cf, h_poly, false, st));
         ZKB_CUDA(cudaStreamSynchronize(st));
     }
-    int next_id = 0;   // identities of the committed polynomials, in this order
+    const uint32_t nc = p.nc, na = cs.na, ns = pk->nsets;
+    int next_id = 0;   // identities of the committed polynomials, in this order; per-circuit ones circuit-major
     auto ids = [&](size_t count) { std::vector<int> v(count); for (auto &e : v) e = next_id++; return v; };
-    const std::vector<int> adv_id = ids(cs.na), fix_id = ids(cs.nf), sig_id = ids(cs.perm.size()), z_id = ids(pk->nsets), phi_id = ids(nl), m_id = ids(nl);
+    const std::vector<int> adv_id = ids(nc * na), fix_id = ids(cs.nf), sig_id = ids(cs.perm.size()), z_id = ids(nc * ns), phi_id = ids(nc * nl),
+                           m_id = ids(nc * nl);
     const int h_id = next_id++, rand_id = next_id++;
     const int64_t rot_last = -(int64_t)(p.bf + 1);
-    // (1) the evaluations written to the transcript, in order; the queries are built afterwards in the multiopen order
+    // (1) the evaluations written to the transcript, in order: every circuit's advice queries, the fixed queries, the random
+    // polynomial, sigma, every circuit's z evaluations, every circuit's lookup evaluations; the queries are built afterwards in
+    // the multiopen order
     struct EvalReq { int poly_id; const Fr *poly; int64_t rot; };
     std::vector<EvalReq> reqs;
-    for (auto &q : cs.advq) reqs.push_back({adv_id[q[0]], p.adv_polys[q[0]], q[1]});
+    for (uint32_t c = 0; c < nc; ++c)
+        for (auto &q : cs.advq) reqs.push_back({adv_id[c * na + q[0]], p.adv_polys[c * na + q[0]], q[1]});
     for (auto &q : cs.fixq) reqs.push_back({fix_id[q[0]], pk->fixed_polys[q[0]], q[1]});
     reqs.push_back({rand_id, p.random_poly, 0});
     for (size_t i = 0; i < cs.perm.size(); ++i) reqs.push_back({sig_id[i], pk->sigma_polys[i], 0});
-    for (uint32_t i = 0; i < pk->nsets; ++i) {
-        reqs.push_back({z_id[i], p.z_polys[i], 0});
-        reqs.push_back({z_id[i], p.z_polys[i], 1});
-        if (i + 1 != pk->nsets) reqs.push_back({z_id[i], p.z_polys[i], rot_last});
+    for (uint32_t u = 0; u < nc * ns; ++u) {
+        reqs.push_back({z_id[u], p.z_polys[u], 0});
+        reqs.push_back({z_id[u], p.z_polys[u], 1});
+        if (u % ns + 1 != ns) reqs.push_back({z_id[u], p.z_polys[u], rot_last});
     }
-    for (size_t l = 0; l < nl; ++l) {
-        reqs.push_back({phi_id[l], p.phi_polys[l], 0});
-        reqs.push_back({phi_id[l], p.phi_polys[l], 1});
-        reqs.push_back({m_id[l], p.m_polys[l], 0});
+    for (size_t u = 0; u < nc * nl; ++u) {
+        reqs.push_back({phi_id[u], p.phi_polys[u], 0});
+        reqs.push_back({phi_id[u], p.phi_polys[u], 1});
+        reqs.push_back({m_id[u], p.m_polys[u], 0});
     }
     const size_t n_written = reqs.size();
     reqs.push_back({h_id, h_poly, 0});  // needed by SHPLONK, not written
@@ -1583,12 +1652,16 @@ static int32_t evaluate(ProofState &p) {
     for (size_t i = 0; i < n_written; ++i) p.s->tr.write_scalar(evals[i]);
     for (size_t i = 0; i < reqs.size(); ++i) p.eval_of[{reqs[i].poly_id, reqs[i].rot}] = evals[i];
 
-    // (2) multiopen queries in prover.rs order
+    // (2) multiopen queries in prover.rs order: per circuit [advice; z at x, omega x per set, then z at omega^last x for the sets
+    // in reverse, skipping the last; lookups], then fixed, sigma, h, random
     auto push_q = [&](int id, const Fr *poly, int64_t rot) { p.queries.push_back({id, poly, rot, p.point_of[rot], p.eval_of[{id, rot}]}); };
-    for (auto &q : cs.advq) push_q(adv_id[q[0]], p.adv_polys[q[0]], q[1]);
-    for (uint32_t i = 0; i < pk->nsets; ++i) { push_q(z_id[i], p.z_polys[i], 0); push_q(z_id[i], p.z_polys[i], 1); }
-    for (int i = (int)pk->nsets - 2; i >= 0; --i) push_q(z_id[i], p.z_polys[i], rot_last);
-    for (size_t l = 0; l < nl; ++l) { push_q(phi_id[l], p.phi_polys[l], 0); push_q(phi_id[l], p.phi_polys[l], 1); push_q(m_id[l], p.m_polys[l], 0); }
+    for (uint32_t c = 0; c < nc; ++c) {
+        for (auto &q : cs.advq) push_q(adv_id[c * na + q[0]], p.adv_polys[c * na + q[0]], q[1]);
+        const uint32_t z0 = c * ns;
+        for (uint32_t i = z0; i < z0 + ns; ++i) { push_q(z_id[i], p.z_polys[i], 0); push_q(z_id[i], p.z_polys[i], 1); }
+        for (int i = (int)ns - 2; i >= 0; --i) push_q(z_id[z0 + i], p.z_polys[z0 + i], rot_last);
+        for (size_t l = c * nl; l < (c + 1) * nl; ++l) { push_q(phi_id[l], p.phi_polys[l], 0); push_q(phi_id[l], p.phi_polys[l], 1); push_q(m_id[l], p.m_polys[l], 0); }
+    }
     for (auto &q : cs.fixq) push_q(fix_id[q[0]], pk->fixed_polys[q[0]], q[1]);
     for (size_t i = 0; i < cs.perm.size(); ++i) push_q(sig_id[i], pk->sigma_polys[i], 0);
     push_q(h_id, h_poly, 0);

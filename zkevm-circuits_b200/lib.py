@@ -77,6 +77,7 @@ SIGNATURES = {
     "zkb_prove_begin": (ctypes.c_int32, [_vp, _vp, _vp, _vp, ctypes.POINTER(_vp)]),
     "zkb_prove_begin_ex": (ctypes.c_int32, [_vp, ctypes.c_int32, _vp, _vp, _vp, ctypes.POINTER(_vp)]),
     "zkb_prove_begin_cb": (ctypes.c_int32, [_vp, _vp, _vp, _vp, _vp, ctypes.POINTER(_vp)]),
+    "zkb_prove_begin_multi": (ctypes.c_int32, [_vp, ctypes.c_int32, _vp, _vp, ctypes.c_uint32, _vp, _vp, ctypes.POINTER(_vp)]),
     "zkb_poseidon_hash_host": (ctypes.c_int32, [_vp, ctypes.c_uint64, _vp]),
     "zkb_blake2b_challenge_host": (ctypes.c_int32, [_vp, ctypes.c_uint64, _vp]),
     "zkb_keccak256_host": (ctypes.c_int32, [_vp, ctypes.c_uint64, _vp]),

@@ -237,7 +237,7 @@ def create_proof(pk, transcript_repr, instances, synthesize, z_blinds, phi_blind
       where challenges is a dict {index: uint64[4]} of the challenges available so far (Circuit::synthesize stand-in).
     z_blinds (n_sets*bf, 4), phi_blinds (n_lookups*bf, 4), random_poly (n, 4): uint64 Montgomery arrays.
     Returns the proof bytes."""
-    cs, lib, ctx = pk.cs, pk.ctx.lib, pk.ctx
+    lib = pk.ctx.lib
     tr = np.ascontiguousarray(np.asarray(transcript_repr, dtype=np.uint64).reshape(4))
     ki, itbl = _ptr_array(instances)
     lens = (ctypes.c_uint32 * max(1, len(instances)))(*[a.shape[0] for a in instances])
@@ -247,15 +247,48 @@ def create_proof(pk, transcript_repr, instances, synthesize, z_blinds, phi_blind
                                      ctypes.cast(lens, _vp), ctypes.byref(sess)))
     else:
         check(lib.zkb_prove_begin_ex(pk.handle, TRANSCRIPTS[transcript], _vp(tr.ctypes.data), ctypes.cast(itbl, _vp), ctypes.cast(lens, _vp), ctypes.byref(sess)))
+    return _prove(pk, sess, 1, lambda c, phase, ch: synthesize(phase, ch), z_blinds, phi_blinds, random_poly, upload_ahead)
+
+
+def create_proof_multi(pk, transcript_repr, instances, synthesize, z_blinds, phi_blinds, random_poly, transcript="blake2b", upload_ahead=False):
+    """Mirror of plonk::create_proof with several circuits (`circuits: &[C]`, `instances: &[&[&[Fr]]]`): ONE proof of C circuits of
+    the same constraint system.  They share the challenges, one quotient and one SHPLONK opening (zkb_prove_begin_multi).
+
+    instances: one list per circuit of uint64 (len, 4) arrays (one per instance column).
+    synthesize(circuit, phase, challenges) -> dict {advice column: uint64 (n,4) array, already blinded} for circuit `circuit`.
+    z_blinds (C*n_sets*bf, 4) and phi_blinds (C*n_lookups*bf, 4): circuit-major; random_poly (n, 4): one for the proof.
+    transcript and upload_ahead as in create_proof.  Returns the proof bytes (empty with a CallbackTranscript)."""
+    cs, lib = pk.cs, pk.ctx.lib
+    nc = len(instances)
+    for inst in instances:
+        assert len(inst) == cs.num_instance, "every circuit passes one array per instance column"
+    tr = np.ascontiguousarray(np.asarray(transcript_repr, dtype=np.uint64).reshape(4))
+    flat = [a for inst in instances for a in inst]
+    ki, itbl = _ptr_array(flat)
+    lens = (ctypes.c_uint32 * max(1, len(flat)))(*[a.shape[0] for a in flat])
+    cb = isinstance(transcript, CallbackTranscript)
+    vt = ctypes.cast(ctypes.pointer(transcript.vt), _vp) if cb else None
+    sess = _vp()
+    check(lib.zkb_prove_begin_multi(pk.handle, 3 if cb else TRANSCRIPTS[transcript], vt, _vp(tr.ctypes.data), nc, ctypes.cast(itbl, _vp),
+                                    ctypes.cast(lens, _vp), ctypes.byref(sess)))
+    return _prove(pk, sess, nc, synthesize, z_blinds, phi_blinds, random_poly, upload_ahead)
+
+
+def _prove(pk, sess, nc, synthesize, z_blinds, phi_blinds, random_poly, upload_ahead):
+    """the advice phases and zkb_prove_finish of a begun session of nc circuits; destroys the session"""
+    cs, lib = pk.cs, pk.ctx.lib
+    na = cs.num_advice
     try:
         nch = len(cs.challenge_phase)
         ch_buf = np.zeros((max(1, nch), 4), dtype=np.uint64)
         challenges = {}
         for phase in range(cs.num_phases()):
-            cols = synthesize(phase, dict(challenges))
-            arrs = [cols.get(c) if cs.advice_phase[c] == phase else None for c in range(cs.num_advice)]
-            for c, a in enumerate(arrs):
-                if cs.advice_phase[c] == phase:
+            arrs = []      # circuit-major: circuit c's column j at c * na + j
+            for circ in range(nc):
+                cols = synthesize(circ, phase, dict(challenges))
+                arrs += [cols.get(c) if cs.advice_phase[c] == phase else None for c in range(na)]
+            for i, a in enumerate(arrs):
+                if cs.advice_phase[i % na] == phase:
                     assert a is not None and a.shape == (cs.n, 4) and a.dtype == np.uint64
             if upload_ahead:   # column by column ahead of the phase call (zkb_prove_upload_advice), then NULL pointers in the phase call
                 idx = [c for c, a in enumerate(arrs) if a is not None]
